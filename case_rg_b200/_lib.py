@@ -40,7 +40,7 @@ class SelectArgs(C.Structure):
     _fields_ = [(n, i32) for n in ('mode', 'B', 'W', 't', 'max_len', 'Tmax', 'BOS', 'EOS', 'UNK', 'PAD')] + \
                [(n, vp) for n in ('top_vals', 'top_idx', 'live', 'cum', 'length', 'tok', 'anc_in', 'anc_out',
                                   'parent', 'ended', 'best_key', 'best_len', 'out_tokens', 'n_live')] + \
-               [('V_in', i32), ('tok_ext', vp)]
+               [('V_in', i32), ('tok_ext', vp), ('nbest', i32)]
 
 
 class PostLinear(C.Structure):
@@ -75,7 +75,7 @@ class StepArgs(C.Structure):
                 ('out_tokens', vp), ('n_live', vp),
                 ('x_in', vp), ('h', vp), ('bbuf', vp), ('q2', vp), ('part_ml', vp), ('part_acc', vp), ('qa', vp),
                 ('attn_un', vp * 2), ('stats', vp * 2), ('ctxp', vp * 2), ('hN', vp), ('ctx', vp * 2), ('gates', vp),
-                ('fac', vp), ('gfeat', vp), ('logits', vp), ('dist', vp), ('top_vals', vp), ('top_idx', vp), ('vocab_ws', vp), ('prow', vp), ('h0', vp), ('qa1', vp), ('base_ms', vp), ('base_e', vp), ('base_i', vp), ('xcount', vp), ('xprefix', vp), ('xslots', i32), ('xidx', vp), ('xorder', vp), ('qcount', vp), ('Wqa_c', vp * 2), ('Wg_c', vp), ('xns', vp), ('cp_n', vp), ('cp_uid', vp), ('cp_first', vp), ('cp_start', vp), ('cp_perm', vp), ('cp_ld', i32), ('Gv', vp * 2), ('opt', i32), ('fork', vp), ('n_oov', i32), ('tok_ext', vp)]
+                ('fac', vp), ('gfeat', vp), ('logits', vp), ('dist', vp), ('top_vals', vp), ('top_idx', vp), ('vocab_ws', vp), ('prow', vp), ('h0', vp), ('qa1', vp), ('base_ms', vp), ('base_e', vp), ('base_i', vp), ('xcount', vp), ('xprefix', vp), ('xslots', i32), ('xidx', vp), ('xorder', vp), ('qcount', vp), ('Wqa_c', vp * 2), ('Wg_c', vp), ('xns', vp), ('cp_n', vp), ('cp_uid', vp), ('cp_first', vp), ('cp_start', vp), ('cp_perm', vp), ('cp_ld', i32), ('Gv', vp * 2), ('opt', i32), ('fork', vp), ('n_oov', i32), ('tok_ext', vp), ('nbest', i32)]
 
 
 class GttpStepArgs(C.Structure):
@@ -90,7 +90,7 @@ class GttpStepArgs(C.Structure):
                                   'out_tokens', 'n_live', 'emb', 'qa')] + \
                [('attn_un', vp * 2), ('stats', vp * 2), ('ctxp', vp * 2), ('ctx', vp * 2)] + \
                [(n, vp) for n in ('gi', 'gh', 'feat', 'gates', 'fac', 'logits', 'dist', 'top_vals', 'top_idx', 'vocab_ws')] + \
-               [('opt', i32)] + [(n, vp) for n in ('base_ms', 'base_e', 'base_i', 'fork', 'qa1')]
+               [('opt', i32)] + [(n, vp) for n in ('base_ms', 'base_e', 'base_i', 'fork', 'qa1')] + [('nbest', i32)]
 
 
 # name -> argtypes (return type is int for all but the three listed below)

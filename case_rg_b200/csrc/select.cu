@@ -28,6 +28,8 @@ extern "C" int case_beam_select(const case_select_args_t* a, case_stream_t strea
              "case_beam_select: null pointer");
   CB_REQUIRE(a->B > 0 && a->W >= 1 && a->W <= CASE_MAX_W && a->t >= 0 && a->t < a->max_len && a->max_len <= a->Tmax,
              "case_beam_select: bad sizes");
+  const int rc = check_nbest(a->nbest, a->W, a->mode);
+  if (rc) return rc;
   if (a->mode == CASE_MODE_BEAM) {
     CB_REQUIRE(a->top_vals && a->cum && a->length && a->anc_in && a->best_key && a->best_len,
                "case_beam_select: beam mode needs top_vals/cum/length/anc_in/best_*");

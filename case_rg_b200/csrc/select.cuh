@@ -6,6 +6,14 @@
 
 namespace cb {
 
+// The n-best list (case_select_args_t.nbest) holds at most W <= CASE_MAX_W entries and exists in beam mode only; every
+// launcher that can run the select checks it before its first launch.
+static inline int check_nbest(int nbest, int W, int mode) {
+  CB_REQUIRE(nbest >= 0 && nbest <= W && nbest <= CASE_MAX_W, "nbest out of range: 0 <= nbest <= W <= CASE_MAX_W");
+  CB_REQUIRE(nbest <= 1 || mode == CASE_MODE_BEAM, "nbest > 1 needs CASE_MODE_BEAM");
+  return 0;
+}
+
 // One warp runs the bookkeeping of query b (all 32 lanes must call).  top_vals / top_idx may have been
 // written by other CTAs of the same launch (fused form: the last CTA of the query's W rows calls this
 // after a fence + atomic), hence the L2 (.cg) loads.
@@ -38,9 +46,15 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
     return;
   }
 
-  __shared__ double key[64], ccum[64];
-  __shared__ int ctok[64], cpar[64], clen[64], order[CASE_MAX_W], dst[CASE_MAX_W];
-  __shared__ int s_nlive, s_best;
+  // n-best list of the query, in rank order: keys bkey, lengths blen, token rows out[i] ([nb][Tmax])
+  const int nb = a.nbest > 1 ? a.nbest : 1;
+  double* bkey = a.best_key + (size_t)b * nb;
+  int32_t* blen = a.best_len + (size_t)b * nb;
+  int* out = a.out_tokens + (size_t)b * nb * a.Tmax;
+  __shared__ double key[64], ccum[64], s_bkey[CASE_MAX_W];
+  __shared__ int ctok[64], cpar[64], clen[64], order[CASE_MAX_W], dst[CASE_MAX_W], ins[CASE_MAX_W], s_blen[CASE_MAX_W];
+  __shared__ int s_nlive;
+  if (lane < nb) { s_bkey[lane] = bkey[lane]; s_blen[lane] = blen[lane]; }
   int nl = 0;
   for (int w = 0; w < W; ++w) nl += a.live[r0 + w] != 0;
   const int ncand = nl * W;
@@ -66,24 +80,32 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
   __syncwarp();
   const int nsel = min(W, ncand);
   if (lane == 0) {
-    int nn = 0, bc = -1;
-    double bk = a.best_key[b];
+    int nn = 0;
     for (int k = 0; k < nsel; ++k) {
       const int c = order[k];
       const bool fin = (ctok[c] == a.EOS) || (t == a.max_len - 1);   // Generations.py:139
+      ins[k] = -1;
       if (fin) {
-        if (key[c] < bk) { bk = key[c]; bc = c; }                     // first finisher wins ties (:184)
+        // stable sort of the finished list (:183-185): after every entry whose key is <= this one, so equal keys stay
+        // in finishing order; a position >= nb drops it (nb = 1: the first finisher wins ties)
+        int pos = 0;
+        while (pos < nb && s_bkey[pos] <= key[c]) ++pos;
+        if (pos < nb) {
+          for (int i = nb - 1; i > pos; --i) { s_bkey[i] = s_bkey[i - 1]; s_blen[i] = s_blen[i - 1]; }
+          s_bkey[pos] = key[c];
+          s_blen[pos] = t + 1;
+          ins[k] = pos;
+        }
         dst[k] = -1;
       } else {
         dst[k] = nn++;
       }
     }
     s_nlive = nn;
-    s_best = bc;
-    if (bc >= 0) a.best_key[b] = bk;
     a.n_live[b] = nn;
   }
   __syncwarp();
+  if (lane < nb) { bkey[lane] = s_bkey[lane]; blen[lane] = s_blen[lane]; }
   // read everything the new slots need from the old state before any slot is overwritten
   // (anc is double-buffered; cum/length/live were staged in shared memory above)
   for (int k = 0; k < nsel; ++k) {
@@ -108,10 +130,14 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
     if (ext) tok_o[(size_t)rn * TL + t + 1] = a.PAD;
     for (int j = 0; j <= t; ++j) a.anc_out[(size_t)rn * TL + j] = rn;
   }
-  if (s_best >= 0) {   // record the new best finished sequence: BOS dropped, EOS kept (:188)
-    const int c = s_best, pr = cpar[c];
-    int* out = a.out_tokens + (size_t)b * a.Tmax;
+  // record the inserted finished sequences in insertion order: BOS dropped, EOS kept (:188).  Lane j owns column j of
+  // every row, so the shift of the lower rows and the new row need no synchronisation between insertions.
+  for (int k = 0; k < nsel; ++k) {
+    const int pos = ins[k];
+    if (pos < 0) continue;
+    const int c = order[k], pr = cpar[c];
     for (int j = lane; j < a.max_len; j += 32) {
+      for (int i = nb - 1; i > pos; --i) out[(size_t)i * a.Tmax + j] = out[(size_t)(i - 1) * a.Tmax + j];
       int v = a.PAD;
       if (j < t) {
         const int src = (j + 1 == t) ? pr : a.anc_in[(size_t)pr * TL + j + 1];
@@ -119,9 +145,8 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
       } else if (j == t) {
         v = ctok[c];
       }
-      out[j] = v;
+      out[(size_t)pos * a.Tmax + j] = v;
     }
-    if (lane == 0) a.best_len[b] = t + 1;
   }
 }
 

@@ -566,6 +566,10 @@ extern "C" int case_sparse_tail(const case_tail_args_t* a, const float* base_ms,
   // plan mode: (id, value) per list entry, at most one per source position; the hash layout otherwise
   const size_t smem = plan ? (size_t)((total + 3) / 4 * 4) * 8 : (size_t)nslots * 12;
   if (plan) nslots = (total + 3) / 4 * 4;
+  if (sel) {
+    const int rc = check_nbest(sel->nbest, sel->W, sel->mode);
+    if (rc) return rc;
+  }
   cudaStream_t st = (cudaStream_t)stream;
   ensure_smem<sparse_tail_kernel>(16384 * 12);
   CB_REQUIRE(sel == nullptr || (qcount != nullptr && sel->B * sel->W == a->R && sel->W == a->W && a->K == a->W),

@@ -5,6 +5,7 @@
 #include <string.h>
 
 #include "common.cuh"
+#include "select.cuh"
 
 namespace cb {
 
@@ -111,28 +112,28 @@ static case_select_args_t select_args(int mode, int B, int W, int t, int max_len
                                       int PAD, const float* top_vals, const int32_t* top_idx, int32_t* live, double* cum,
                                       int32_t* length, int32_t* tok, int32_t* const anc[2], int32_t* parent,
                                       int32_t* ended, double* best_key, int32_t* best_len, int32_t* out_tokens,
-                                      int32_t* n_live) {
+                                      int32_t* n_live, int nbest) {
   case_select_args_t s;
   memset(&s, 0, sizeof(s));
   s.mode = mode; s.B = B; s.W = W; s.t = t; s.max_len = max_len; s.Tmax = Tmax;
   s.BOS = BOS; s.EOS = EOS; s.UNK = UNK; s.PAD = PAD;
   s.top_vals = top_vals; s.top_idx = top_idx; s.live = live; s.cum = cum; s.length = length; s.tok = tok;
   s.anc_in = anc[t & 1]; s.anc_out = anc[(t + 1) & 1]; s.parent = parent; s.ended = ended;
-  s.best_key = best_key; s.best_len = best_len; s.out_tokens = out_tokens; s.n_live = n_live;
+  s.best_key = best_key; s.best_len = best_len; s.out_tokens = out_tokens; s.n_live = n_live; s.nbest = nbest;
   return s;
 }
 
 static int select_step(int mode, int B, int W, int t, int max_len, int Tmax, int BOS, int EOS, int UNK, int PAD,
                        const float* top_vals, const int32_t* top_idx, int32_t* live, double* cum, int32_t* length,
                        int32_t* tok, int32_t* const anc[2], int32_t* parent, int32_t* ended, double* best_key,
-                       int32_t* best_len, int32_t* out_tokens, int32_t* n_live, cudaStream_t st) {
+                       int32_t* best_len, int32_t* out_tokens, int32_t* n_live, int nbest, cudaStream_t st) {
   case_select_args_t s;
   memset(&s, 0, sizeof(s));
   s.mode = mode; s.B = B; s.W = W; s.t = t; s.max_len = max_len; s.Tmax = Tmax;
   s.BOS = BOS; s.EOS = EOS; s.UNK = UNK; s.PAD = PAD;
   s.top_vals = top_vals; s.top_idx = top_idx; s.live = live; s.cum = cum; s.length = length; s.tok = tok;
   s.anc_in = anc[t & 1]; s.anc_out = anc[(t + 1) & 1]; s.parent = parent; s.ended = ended;
-  s.best_key = best_key; s.best_len = best_len; s.out_tokens = out_tokens; s.n_live = n_live;
+  s.best_key = best_key; s.best_len = best_len; s.out_tokens = out_tokens; s.n_live = n_live; s.nbest = nbest;
   return case_beam_select(&s, st);
 }
 
@@ -141,6 +142,7 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
   CB_REQUIRE(a->R == a->B * a->W && a->W >= 1 && a->W <= CASE_MAX_W, "case_decode_step: R != B*W or W out of range");
   CB_REQUIRE(t >= 0 && t < a->Tmax && a->Tmax <= CASE_MAX_T, "case_decode_step: t out of range");
   CB_REQUIRE(a->materialize_only || t < a->max_len, "case_decode_step: t >= max_len");
+  TRY(check_nbest(a->nbest, a->W, a->mode));
   cudaStream_t st = (cudaStream_t)stream;
   const int R = a->R, B = a->B, W = a->W, TL = a->Tmax + 1, dt = a->dtype;
   const int32_t* anc = a->anc[t & 1];
@@ -359,7 +361,7 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
       const bool fuse_sel = a->qcount != nullptr && !(opt & CASE_OPT_NO_FUSED_SELECT);
       case_select_args_t sel = select_args(a->mode, B, W, t, a->max_len, a->Tmax, a->BOS, a->EOS, a->UNK, a->PAD,
                                            a->top_vals, a->top_idx, a->live, a->cum, a->length, a->tok, a->anc, a->parent,
-                                           a->ended, a->best_key, a->best_len, a->out_tokens, a->n_live);
+                                           a->ended, a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
       if (n_oov) { sel.V_in = a->V; sel.tok_ext = a->tok_ext; }
       TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2, fuse_sel ? &sel : nullptr, a->qcount, st));
       if (fuse_sel) return 0;
@@ -383,7 +385,7 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
   {
     case_select_args_t sel = select_args(a->mode, B, W, t, a->max_len, a->Tmax, a->BOS, a->EOS, a->UNK, a->PAD, a->top_vals,
                                          a->top_idx, a->live, a->cum, a->length, a->tok, a->anc, a->parent, a->ended,
-                                         a->best_key, a->best_len, a->out_tokens, a->n_live);
+                                         a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
     if (n_oov) { sel.V_in = a->V; sel.tok_ext = a->tok_ext; }
     return case_beam_select(&sel, st);
   }
@@ -403,6 +405,7 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
   CB_REQUIRE(a, "gttp_decode_step: null args");
   CB_REQUIRE(a->R == a->B * a->W && a->W >= 1 && a->W <= CASE_MAX_W, "gttp_decode_step: R != B*W or W out of range");
   CB_REQUIRE(t >= 0 && t < a->Tmax && a->Tmax <= CASE_MAX_T, "gttp_decode_step: t out of range");
+  TRY(check_nbest(a->nbest, a->W, a->mode));
   cudaStream_t st = (cudaStream_t)stream;
   const int R = a->R, B = a->B, W = a->W, TL = a->Tmax + 1, dt = a->dtype;
   const float* s_in = a->state[t & 1];
@@ -509,7 +512,7 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
   }
   return select_step(a->mode, B, W, t, a->max_len, a->Tmax, a->BOS, a->EOS, a->UNK, a->PAD, a->top_vals, a->top_idx,
                      a->live, a->cum, a->length, a->tok, a->anc, a->parent, a->ended, a->best_key, a->best_len,
-                     a->out_tokens, a->n_live, st);
+                     a->out_tokens, a->n_live, a->nbest, st);
 }
 
 /* layout self-check for FFI bindings: sizeof of each argument struct, by index */

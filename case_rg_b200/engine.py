@@ -14,7 +14,7 @@ Generations.greedy/beam (common/Generations.py:66-190) and the GTTP step (GTTP/M
 import ctypes as C
 import math
 import os
-from typing import Dict, Optional
+from typing import Dict, NamedTuple, Optional
 
 import torch
 
@@ -300,11 +300,36 @@ class CaseWeights:
         self.Wm_g = [self.Wm[:, H * (1 + i):H * (2 + i)].contiguous() for i in range(2)]          # [3][H] each
 
 
-class _SearchState:
-    """Buffers shared by both engines for the on-device greedy / beam bookkeeping."""
+class NBest(NamedTuple):
+    """The n best finished hypotheses of every query, in rank order (sorted(results[q], key=cum_cost/length)[:n],
+    Generations.py:183-185): ``tokens`` int64 [B, n, L] (BOS dropped, EOS kept, zero padded to the longest entry of the
+    batch), ``lengths`` int64 [B, n] answer tokens, ``costs`` fp64 [B, n] the ranking key cum_cost / length in nats per
+    position (BOS counted in the length; lower is better)."""
+    tokens: torch.Tensor
+    lengths: torch.Tensor
+    costs: torch.Tensor
 
-    def __init__(self, dev, B, W, Tmax, ext=False):
+
+def nbest_from(out_tokens, best_len, best_key) -> NBest:
+    """n-best buffers of a search state (out_tokens [B, (n,) Tmax], best_len / best_key [B, (n)]) -> NBest on their
+    device, trimmed like merge1D (Utils.py:366-377) to the longest entry."""
+    B = best_len.size(0)
+    lengths = best_len.reshape(B, -1).to(torch.int64)
+    n = lengths.size(1)
+    L = max(int(lengths.max()), 1)
+    return NBest(out_tokens.reshape(B, n, -1)[:, :, :L].to(torch.int64), lengths,
+                 best_key.reshape(B, n).clone())
+
+
+class _SearchState:
+    """Buffers shared by both engines for the on-device greedy / beam bookkeeping.  nbest > 1: the beam search keeps
+    the nbest best finished hypotheses of every query (best_key / best_len [B, nbest], out_tokens [B, nbest, Tmax])."""
+
+    def __init__(self, dev, B, W, Tmax, ext=False, nbest=1):
+        if not 1 <= nbest <= W:
+            raise ValueError(f'nbest must be 1..{W} (the beam width), got {nbest}')
         R, TL = B * W, Tmax + 1
+        nb = () if nbest == 1 else (nbest,)
         i32 = dict(dtype=torch.int32, device=dev)
         self.tok = torch.zeros(R, TL, **i32)
         # extended vocabulary: tok feeds the decoder (OOV ids become UNK), tok_ext keeps the ids of the returned sequences
@@ -315,11 +340,11 @@ class _SearchState:
         self.length = torch.zeros(R, **i32)
         self.parent = torch.zeros(R, **i32)
         self.ended = torch.zeros(B, **i32)
-        self.best_key = torch.zeros(B, dtype=torch.float64, device=dev)
-        self.best_len = torch.zeros(B, **i32)
-        self.out_tokens = torch.zeros(B, Tmax, **i32)
+        self.best_key = torch.zeros(B, *nb, dtype=torch.float64, device=dev)
+        self.best_len = torch.zeros(B, *nb, **i32)
+        self.out_tokens = torch.zeros(B, *nb, Tmax, **i32)
         self.n_live = torch.zeros(B, **i32)
-        self.B, self.W, self.R, self.Tmax = B, W, R, Tmax
+        self.B, self.W, self.R, self.Tmax, self.nbest = B, W, R, Tmax, nbest
         self._arange = torch.arange(R, **i32)
         self._slot0 = (self._arange % W == 0).to(torch.int32)
 
@@ -344,6 +369,7 @@ class _SearchState:
         a.anc[0], a.anc[1] = self.anc[0].data_ptr(), self.anc[1].data_ptr()
         for n in ('tok', 'live', 'cum', 'length', 'parent', 'ended', 'best_key', 'best_len', 'out_tokens', 'n_live'):
             setattr(a, n, getattr(self, n).data_ptr())
+        a.nbest = self.nbest
 
 
 class _EngineBase:
@@ -388,12 +414,17 @@ class _EngineBase:
 
     def _finish_tokens(self, max_len: int, mode: int) -> torch.Tensor:
         st = self.state
-        out = st.out_tokens[:, :max_len].to(torch.int64)
+        out = st.out_tokens.view(st.B, -1, st.Tmax)[:, 0, :max_len].to(torch.int64)   # entry 0 of an n-best list
         if mode == L.MODE_BEAM:
             # merge1D (Utils.py:366-377): pad to the longest answer of the batch
-            Lmax = int(st.best_len.max().item())
+            Lmax = int(st.best_len.view(st.B, -1)[:, 0].max().item())
             out = out[:, :max(Lmax, 1)]
         return out
+
+    def _finish_nbest(self) -> NBest:
+        """The n-best list of the last beam decode (see NBest), on the engine's device."""
+        st = self.state
+        return nbest_from(st.out_tokens, st.best_len, st.best_key)
 
 
 class CaseDecodeEngine(_EngineBase):
@@ -401,9 +432,10 @@ class CaseDecodeEngine(_EngineBase):
 
     def __init__(self, weights: CaseWeights, B: int, W: int, S0: int, S1: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0, n_oov: int = 0):
+                 opt: int = 0, n_oov: int = 0, nbest: int = 1):
         """n_oov > 0: extended vocabulary - ``source_map`` entries in [V, V + n_oov) are per-query dynamic (OOV) words,
-        the mixture and its top-k range over V + n_oov ids (pointer-generator extension; an OOV id is fed back as UNK)."""
+        the mixture and its top-k range over V + n_oov ids (pointer-generator extension; an OOV id is fed back as UNK).
+        nbest (1..W): a beam decode keeps the nbest best finished hypotheses per query (read with ``_finish_nbest``)."""
         self.opt, self.n_oov = int(opt), int(n_oov)
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
@@ -448,7 +480,7 @@ class CaseDecodeEngine(_EngineBase):
         # state
         self.kcache = [torch.zeros(R, Tmax, H, dtype=td, device=dev) for _ in range(8)]
         self.vcache = [torch.zeros(R, Tmax, H, dtype=td, device=dev) for _ in range(8)]
-        self.state = _SearchState(dev, B, W, Tmax, ext=self.n_oov > 0)
+        self.state = _SearchState(dev, B, W, Tmax, ext=self.n_oov > 0, nbest=nbest)
         # scratch
         # second memory: only valid keys are packed (case_cross_attn_part); CASE_NO_COMPACT=1 keeps the masked form (A/B)
         self.compact = weights.cdtype == L.BF16 and os.environ.get('CASE_NO_COMPACT', '0') != '1'
@@ -670,7 +702,8 @@ class CaseDecodeEngine(_EngineBase):
         return self.dist[:, :self.V + self.n_oov]
 
     def answer_tokens(self) -> int:
-        return int(self.state.best_len.sum().item())
+        st = self.state
+        return int(st.best_len.view(st.B, -1)[:, 0].sum().item())      # entry 0 of an n-best list
 
     def kernel_launches_per_step(self) -> int:
         # (+1 in bench.py: the activation re-pack inside the vocabulary GEMM call)
@@ -717,7 +750,7 @@ class GttpWeights:
 class GttpDecodeEngine(_EngineBase):
     def __init__(self, weights: GttpWeights, B: int, W: int, Lc: int, Lb: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0):
+                 opt: int = 0, nbest: int = 1):
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
         self.w = weights
@@ -740,7 +773,7 @@ class GttpDecodeEngine(_EngineBase):
         self.mask = [torch.zeros(B, s, dtype=torch.uint8, device=dev) for s in (Lc, Lb)]
         self.map = torch.zeros(B, Lb, dtype=torch.int32, device=dev)
         self.gstate = [z(R, H), z(R, H)]
-        self.state = _SearchState(dev, B, W, Tmax)
+        self.state = _SearchState(dev, B, W, Tmax, nbest=nbest)
         self.emb, self.qa = z(R, H), z(R, H)
         self.attn_un = [z(R, Lc), z(R, Lb)]
         self.stats = [z(R, n, 4) for n in self.ns]

@@ -7,6 +7,9 @@ the model's encoder outputs to an engine and return the same LongTensor the refe
 (``[B, max_len]`` for greedy; for beam the best hypothesis per query without BOS, EOS kept,
 zero-padded to the longest answer - ``merge1D``, common/Utils.py:366-377).
 
+``beam_nbest`` returns more than the reference's single answer: the n best finished hypotheses of every query with
+their costs, the sorted ``results[q]`` list that Generations.beam builds and reads element 0 of (Generations.py:183-185).
+
 ``FastCaSE`` gives the unchanged CaSE decoder the protocol the reference never implemented for it
 (SURVEY.md §8c adapter); ``FastGTTP`` replaces ``GTTP.decode/generate/to_word`` + the search
 (GTTP/Model.py:176-193).  Both take the *encoder-side outputs* as inputs: the encoders are outside
@@ -17,7 +20,7 @@ from typing import Dict, Optional
 import torch
 
 from . import _lib as L
-from .engine import CaseDecodeEngine, CaseWeights, GttpDecodeEngine, GttpWeights
+from .engine import CaseDecodeEngine, CaseWeights, GttpDecodeEngine, GttpWeights, NBest, nbest_from
 
 PAD_WORD, BOS_WORD, UNK_WORD, EOS_WORD = '[PAD]', '[unused0]', '[UNK]', '[unused1]'
 
@@ -43,14 +46,35 @@ def beam(model, data, vocab2id=None, max_len=20, width=5, encode_outputs=None, i
     return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states)
 
 
-def beam_batches(model, batches, vocab2id=None, max_len=20, width=5):
+def _nbest_count(n, width):
+    n = width if n is None else int(n)
+    if not 1 <= n <= width:
+        raise ValueError(f'n must be 1..width ({width}), got {n}')
+    return n
+
+
+def beam_nbest(model, data, vocab2id=None, max_len=20, width=5, n=None, encode_outputs=None, init_decoder_states=None):
+    """The n best answers of ``beam`` per query with their costs: ``NBest(tokens, lengths, costs)`` on the model's
+    device, entry [:, i] the i-th of sorted(results[q], key=cum_cost/length)[:n] (Generations.py:183-185).  tokens int64
+    [B, n, L] (BOS dropped, EOS kept, zero padded to the longest entry), lengths int64 [B, n], costs fp64 [B, n] = the
+    ranking key cum_cost / length in nats per position (lower is better).  Entry 0 is what ``beam`` returns.  n defaults
+    to the width; 1 <= n <= width."""
+    _check_vocab(vocab2id)
+    n = _nbest_count(n, width)
+    return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states, nbest=n)
+
+
+def beam_batches(model, batches, vocab2id=None, max_len=20, width=5, n_best=None):
     """``beam`` over an iterable of HOST batches, the way the predict loop feeds a model one batch after
     another (common/CumulativeTrainer.py:141-156): yields the answers of every batch, in order, as host
     LongTensors.  The host-to-device copy of batch i+1 runs on a copy stream while batch i is decoding
     (double-buffered staging, pinned host tensors copy asynchronously), so the PCIe time of the encoder
-    outputs (175 MB per batch at the BASELINE shape) is hidden behind the decode."""
+    outputs (175 MB per batch at the BASELINE shape) is hidden behind the decode.  n_best: yields the ``beam_nbest``
+    lists of every batch instead (NBest of host tensors)."""
     _check_vocab(vocab2id)
-    return model.search_batches(batches, max_len, width, L.MODE_BEAM)
+    if n_best is not None:
+        n_best = _nbest_count(n_best, width)
+    return model.search_batches(batches, max_len, width, L.MODE_BEAM, n_best)
 
 
 def greedy_batches(model, batches, vocab2id=None, max_len=20):
@@ -85,8 +109,8 @@ class _FastModel:
         return to_sentence(batch_indices, self.id2vocab)
 
     # ---- streamed batches (beam_batches / greedy_batches)
-    def search_batches(self, batches, max_len, width, mode):
-        """Generator behind beam_batches / greedy_batches."""
+    def search_batches(self, batches, max_len, width, mode, n_best=None):
+        """Generator behind beam_batches / greedy_batches (n_best: beam mode, yields NBest per batch)."""
         dev = self.weights.device
         main = torch.cuda.current_stream(dev)
         # the copy stream and the two staging sets live as long as the model: allocating 2 x 175 MB on a
@@ -126,7 +150,7 @@ class _FastModel:
             # decoding is never prefilled: engine_for returns the SAME engine for equal shapes, and its decode is
             # ahead of this prefill on the main stream)
             main.wait_event(ready)
-            eng = self._prefill_staged(d, width, max_len)
+            eng = self._prefill_staged(d, width, max_len, n_best or 1)
             prefilled[k] = torch.cuda.Event()
             prefilled[k].record(main)
             nxt = next(it, None)
@@ -138,7 +162,9 @@ class _FastModel:
                 # answers of the previous batch: snapshot them on the device (stream-ordered after its decode), put
                 # THIS batch's decode behind the snapshot right away, and only then wait for the snapshot on a side
                 # stream - the device never idles while the host reads answers
-                snap = (pending.state.out_tokens[:, :max_len].clone(), pending.state.best_len.clone())
+                st = pending.state
+                snap = (st.out_tokens[..., :max_len].clone(), st.best_len.clone()) + \
+                    ((st.best_key.clone(),) if n_best else ())
                 ev = torch.cuda.Event()
                 ev.record(main)
                 eng.launch(max_len, mode, use_graph=self.use_graph)
@@ -148,19 +174,25 @@ class _FastModel:
             self.last_engine = pending = eng
             k ^= 1
         if pending is not None:
-            yield pending._finish_tokens(max_len, mode).cpu()
+            if n_best:
+                yield NBest(*(x.cpu() for x in pending._finish_nbest()))
+            else:
+                yield pending._finish_tokens(max_len, mode).cpu()
 
     def _read_snapshot(self, snap, ev, mode):
-        """Device snapshot (tokens [B, T] int32, best_len [B]) -> host int64 tokens, trimmed like _finish_tokens."""
+        """Device snapshot (tokens [B, T] int32, best_len [B], or with best_key [B, n] the n-best buffers) -> host int64
+        tokens trimmed like _finish_tokens, or the host NBest."""
         dev = self.weights.device
         if getattr(self, '_d2h_stream', None) is None:
             self._d2h_stream = torch.cuda.Stream(dev)
         d2h = self._d2h_stream
         d2h.wait_event(ev)
         with torch.cuda.stream(d2h):
-            toks = snap[0].to('cpu', non_blocking=True)
-            blen = snap[1].to('cpu', non_blocking=True)
+            host = [x.to('cpu', non_blocking=True) for x in snap]
         d2h.synchronize()
+        if len(host) == 3:
+            return nbest_from(*host)
+        toks, blen = host
         out = toks.to(torch.int64)
         if mode == L.MODE_BEAM:             # merge1D (Utils.py:366-377): pad to the longest answer of the batch
             out = out[:, :max(int(blen.max()), 1)]
@@ -191,50 +223,62 @@ class FastCaSE(_FastModel):
             from .producers import CaseProducers
             self.producers = CaseProducers(producers, device=self.weights.device)
 
-    def search_ids(self, data, max_len=None, width=None, mode='beam'):
+    def search_ids(self, data, max_len=None, width=None, mode='beam', n_best=None):
         """CaSE.do_test from token ids (CaSE/Model.py:313-331): ``data`` = {'query' int [B,1,Lq], 'passage' int [B,NP,Lp],
-        'source_map' int [B,S]} -> {'answer': LongTensor, 'rank': [B,NP]} like the reference's forward(data, 'test')."""
+        'source_map' int [B,S]} -> {'answer': LongTensor, 'rank': [B,NP]} like the reference's forward(data, 'test').
+        n_best (beam mode): also 'nbest', the ``beam_nbest`` list of the same search (its entry 0 is 'answer')."""
         if self.producers is None:
             raise RuntimeError('FastCaSE was built without producers=...')
         max_len = self.max_dec_len if max_len is None else max_len
         width = self.beam_width if width is None else width
+        if n_best is not None:
+            if mode != 'beam':
+                raise ValueError('n_best needs mode="beam"')
+            n_best = _nbest_count(n_best, width)
         p = self.producers(data['query'], data['passage'])
         d = dict(mem_q=p['mem_q'], mem_p=p['mem_p'], query=data['query'].to(self.weights.device),
                  passage=data['passage'].to(self.weights.device), prior_q=p['prior_q'], prior_p=p['prior_p'],
                  answer_rep=p['answer_rep'], source_map=data['source_map'].to(self.weights.device))
         m = {'beam': L.MODE_BEAM, 'greedy': L.MODE_PROTO_GREEDY, 'module_greedy': L.MODE_MODULE_GREEDY}[mode]
-        return {'answer': self.fast_search(d, max_len, width, m), 'rank': p['rank']}
+        if n_best is None:
+            return {'answer': self.fast_search(d, max_len, width, m), 'rank': p['rank']}
+        nb = self.fast_search(d, max_len, width, m, nbest=n_best)
+        return {'answer': self.last_engine._finish_tokens(max_len, m), 'rank': p['rank'], 'nbest': nb}
 
-    def engine_for(self, B, W, S0, S1, T):
-        key = (B, W, S0, S1, T, self.opt, self.n_oov)
+    def engine_for(self, B, W, S0, S1, T, nbest=1):
+        key = (B, W, S0, S1, T, self.opt, self.n_oov, nbest)
         if key not in self._engines:
             if len(self._engines) >= 4:
                 self._engines.clear()
             self._engines[key] = CaseDecodeEngine(self.weights, B, W, S0, S1, T, vocab_impl=self.vocab_impl,
-                                                  opt=self.opt, n_oov=self.n_oov)
+                                                  opt=self.opt, n_oov=self.n_oov, nbest=nbest)
         return self._engines[key]
 
     def encode(self, data):
         return data
 
-    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None):
+    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None):
+        """-> the answers (LongTensor), or with nbest the NBest list of a beam search."""
         d = encode_outputs if encode_outputs is not None else data
         B = d['source_map'].size(0)
         S0 = d['mem_q'].reshape(B, -1, L.H).size(1)
         S1 = d['mem_p'].reshape(B, -1, L.H).size(1)
-        eng = self.engine_for(B, width, S0, S1, max_len)
+        eng = self.engine_for(B, width, S0, S1, max_len, nbest or 1)
         eng.prefill(d['mem_q'], d['mem_p'], d['query'].ne(0), d['passage'].ne(0), d['prior_q'], d['prior_p'],
                     d['answer_rep'], d['source_map'])
         self.last_engine = eng
-        return eng.decode(max_len, mode, use_graph=self.use_graph)
+        if nbest is None:
+            return eng.decode(max_len, mode, use_graph=self.use_graph)
+        eng.launch(max_len, mode, use_graph=self.use_graph)
+        return eng._finish_nbest()
 
     _KEYS = ('mem_q', 'mem_p', 'query', 'passage', 'prior_q', 'prior_p', 'answer_rep', 'source_map')
 
-    def _prefill_staged(self, d, width, max_len):
+    def _prefill_staged(self, d, width, max_len, nbest=1):
         B = d['source_map'].size(0)
         S0 = d['mem_q'].reshape(B, -1, L.H).size(1)
         S1 = d['mem_p'].reshape(B, -1, L.H).size(1)
-        eng = self.engine_for(B, width, S0, S1, max_len)
+        eng = self.engine_for(B, width, S0, S1, max_len, nbest)
         eng.prefill(d['mem_q'], d['mem_p'], d['query'].ne(0), d['passage'].ne(0), d['prior_q'], d['prior_p'],
                     d['answer_rep'], d['source_map'])
         return eng
@@ -256,31 +300,35 @@ class FastGTTP(_FastModel):
         self.opt = int(opt)
         self._engines = {}
 
-    def engine_for(self, B, W, Lc, Lb, T):
-        key = (B, W, Lc, Lb, T)
+    def engine_for(self, B, W, Lc, Lb, T, nbest=1):
+        key = (B, W, Lc, Lb, T, nbest)
         if key not in self._engines:
             if len(self._engines) >= 4:
                 self._engines.clear()
             self._engines[key] = GttpDecodeEngine(self.weights, B, W, Lc, Lb, T, vocab_impl=self.vocab_impl,
-                                                  opt=self.opt)
+                                                  opt=self.opt, nbest=nbest)
         return self._engines[key]
 
-    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None):
+    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None):
+        """-> the answers (LongTensor), or with nbest the NBest list of a beam search."""
         d = dict(data)
         if encode_outputs is not None:
             d.update(encode_outputs)
         if init_decoder_states is not None:
             d['init_state'] = init_decoder_states
-        eng = self._prefill_staged(d, width, max_len)
+        eng = self._prefill_staged(d, width, max_len, nbest or 1)
         self.last_engine = eng
-        return eng.decode(max_len, mode, use_graph=self.use_graph)
+        if nbest is None:
+            return eng.decode(max_len, mode, use_graph=self.use_graph)
+        eng.launch(max_len, mode, use_graph=self.use_graph)
+        return eng._finish_nbest()
 
     _KEYS = ('context', 'background', 'background_map', 'src_output', 'bg_output', 'init_state')
 
-    def _prefill_staged(self, d, width, max_len):
+    def _prefill_staged(self, d, width, max_len, nbest=1):
         B, Lc = d['context'].shape
         Lb = d['background'].size(1)
-        eng = self.engine_for(B, width, Lc, Lb, max_len)
+        eng = self.engine_for(B, width, Lc, Lb, max_len, nbest)
         eng.prefill(d['src_output'], d['bg_output'], d['context'], d['background'], d['background_map'],
                     d['init_state'])
         return eng

@@ -432,6 +432,12 @@ typedef struct {
    * V_in = 0 / tok_ext = NULL: no extension (tok holds both). */
   int32_t V_in;
   int32_t* tok_ext;
+  /* n-best list (beam mode, 1 <= nbest <= W): the nbest best finished hypotheses of every query instead of the best one,
+   * i.e. sorted(results[q], key=cum_cost/length)[:nbest] of Generations.py:183-185 - keys ascending, equal keys in
+   * finishing order (earlier step first, then the better rank within a step).  best_key [B][nbest] (+inf initially),
+   * best_len [B][nbest] and out_tokens [B][nbest][Tmax] (PAD initially) hold the entries in rank order; entry 0 is the
+   * answer of nbest = 1.  0 or 1: the single best, layouts as above. */
+  int32_t nbest;
 } case_select_args_t;
 
 int case_beam_select(const case_select_args_t* a, case_stream_t stream);
@@ -571,6 +577,7 @@ typedef struct {
    * fed back as UNK and kept in tok_ext [R][Tmax+1] for the output.  n_oov = 0: off. */
   int32_t n_oov;
   int32_t* tok_ext;
+  int32_t nbest;                        /* n-best list of the beam search (case_select_args_t.nbest); 0 or 1: the best only */
 } case_step_args_t;
 
 /* Enqueue one full decode step t (embedding .. select) for all R rows: the body of the eval loop
@@ -604,6 +611,7 @@ typedef struct {
   /* optional: with a fork handle and a second query buffer qa1 [R][H] the attention over the context memory runs on the
    * handle's side stream beside the attention over the background (CASE_OPT_NO_FORK switches it off) */
   case_fork_t* fork; float* qa1;
+  int32_t nbest;                                         /* n-best list of the beam search (case_select_args_t.nbest) */
 } gttp_step_args_t;
 
 /* One GTTP decode step (GTTP/Model.py:176-193 -> BBCDecoder.forward :113-131 ->
