@@ -36,11 +36,25 @@ class LayerWeights(C.Structure):
                                   'W2_t', 'b2', 'ln1_g', 'ln1_b', 'ln2_g', 'ln2_b', 'ln3_g', 'ln3_b', 'Wc')]
 
 
+class Attr(C.Structure):
+    """case_attr_t: the attribution record of one answer token (16 bytes)."""
+    _fields_ = [('part', C.c_float * 3), ('source', i32)]
+
+
+# The attribution pointers trail the argument blocks (ABI version 2 unchanged).  They are appended the ctypes way, by
+# subclassing: SelectArgs / StepArgs / GttpStepArgs keep the fields up to nbest, and the *AttrArgs subclasses add the
+# attribution pointers - the complete blocks the launchers read, and what the engines pass.
+
+
 class SelectArgs(C.Structure):
     _fields_ = [(n, i32) for n in ('mode', 'B', 'W', 't', 'max_len', 'Tmax', 'BOS', 'EOS', 'UNK', 'PAD')] + \
                [(n, vp) for n in ('top_vals', 'top_idx', 'live', 'cum', 'length', 'tok', 'anc_in', 'anc_out',
                                   'parent', 'ended', 'best_key', 'best_len', 'out_tokens', 'n_live')] + \
                [('V_in', i32), ('tok_ext', vp), ('nbest', i32)]
+
+
+class SelectAttrArgs(SelectArgs):
+    _fields_ = [('attr_cand', vp), ('attr_hist', vp), ('out_attr', vp)]
 
 
 class PostLinear(C.Structure):
@@ -59,7 +73,8 @@ class TailArgs(C.Structure):
                 ('logits', vp), ('hN', vp), ('stats', vp * 2), ('ctxp', vp * 2), ('Wm', vp), ('bm', vp),
                 ('ctx', vp * 2), ('gates', vp), ('fac', vp), ('map', vp), ('prior', vp * 2), ('attn_un', vp * 2),
                 ('top_vals', vp), ('top_idx', vp), ('dist', vp), ('gate_ctx', i32), ('cp_ld', i32),
-                ('cp_n', vp), ('cp_uid', vp), ('cp_first', vp), ('cp_start', vp), ('cp_perm', vp), ('Vext', i32)]
+                ('cp_n', vp), ('cp_uid', vp), ('cp_first', vp), ('cp_start', vp), ('cp_perm', vp), ('Vext', i32),
+                ('attr', vp)]
 
 
 class StepArgs(C.Structure):
@@ -78,6 +93,10 @@ class StepArgs(C.Structure):
                 ('fac', vp), ('gfeat', vp), ('logits', vp), ('dist', vp), ('top_vals', vp), ('top_idx', vp), ('vocab_ws', vp), ('prow', vp), ('h0', vp), ('qa1', vp), ('base_ms', vp), ('base_e', vp), ('base_i', vp), ('xcount', vp), ('xprefix', vp), ('xslots', i32), ('xidx', vp), ('xorder', vp), ('qcount', vp), ('Wqa_c', vp * 2), ('Wg_c', vp), ('xns', vp), ('cp_n', vp), ('cp_uid', vp), ('cp_first', vp), ('cp_start', vp), ('cp_perm', vp), ('cp_ld', i32), ('Gv', vp * 2), ('opt', i32), ('fork', vp), ('n_oov', i32), ('tok_ext', vp), ('nbest', i32)]
 
 
+class StepAttrArgs(StepArgs):
+    _fields_ = [('attr_cand', vp), ('attr_hist', vp), ('out_attr', vp)]
+
+
 class GttpStepArgs(C.Structure):
     _fields_ = [(n, i32) for n in ('B', 'W', 'R', 'V', 'ldv', 'dtype', 'fast_tanh', 'vocab_impl', 'mode', 'Lc', 'Lb',
                                    'nsplit_c', 'nsplit_b', 'max_len', 'BOS', 'EOS', 'UNK', 'PAD',
@@ -91,6 +110,10 @@ class GttpStepArgs(C.Structure):
                [('attn_un', vp * 2), ('stats', vp * 2), ('ctxp', vp * 2), ('ctx', vp * 2)] + \
                [(n, vp) for n in ('gi', 'gh', 'feat', 'gates', 'fac', 'logits', 'dist', 'top_vals', 'top_idx', 'vocab_ws')] + \
                [('opt', i32)] + [(n, vp) for n in ('base_ms', 'base_e', 'base_i', 'fork', 'qa1')] + [('nbest', i32)]
+
+
+class GttpStepAttrArgs(GttpStepArgs):
+    _fields_ = [('attr_cand', vp), ('attr_hist', vp), ('out_attr', vp)]
 
 
 # name -> argtypes (return type is int for all but the three listed below)
@@ -152,7 +175,7 @@ _PROTOS = {
 _SIZE_FNS = ['case_vocab_tc_workspace_bytes', 'case_vocab_tc_packed_weight_bytes']
 _SIZE_FNS2 = ['case_interaction_smem_bytes', 'case_gemm_rows_packed_weight_bytes']      # (int, int) -> size_t
 EXPORTS = sorted(list(_PROTOS) + ['case_abi_version', 'case_last_error', 'case_struct_size'] + _SIZE_FNS + _SIZE_FNS2)
-_STRUCTS = [Seg, RowLinArgs, LayerWeights, SelectArgs, StepArgs, GttpStepArgs, TailArgs, ChainPost]
+_STRUCTS = [Seg, RowLinArgs, LayerWeights, SelectAttrArgs, StepAttrArgs, GttpStepAttrArgs, TailArgs, ChainPost]
 
 _lib = None
 

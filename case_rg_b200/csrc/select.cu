@@ -13,10 +13,11 @@
 
 namespace cb {
 
+template <bool ATTR>
 __global__ __launch_bounds__(32) void beam_select_kernel(case_select_args_t a) {
   pdl_trigger();
   pdl_wait();
-  beam_select_query(a, blockIdx.x, threadIdx.x);
+  beam_select_query<ATTR>(a, blockIdx.x, threadIdx.x);
 }
 
 }  // namespace cb
@@ -28,7 +29,9 @@ extern "C" int case_beam_select(const case_select_args_t* a, case_stream_t strea
              "case_beam_select: null pointer");
   CB_REQUIRE(a->B > 0 && a->W >= 1 && a->W <= CASE_MAX_W && a->t >= 0 && a->t < a->max_len && a->max_len <= a->Tmax,
              "case_beam_select: bad sizes");
-  const int rc = check_nbest(a->nbest, a->W, a->mode);
+  int rc = check_nbest(a->nbest, a->W, a->mode);
+  if (rc) return rc;
+  rc = check_attr_select(*a);
   if (rc) return rc;
   if (a->mode == CASE_MODE_BEAM) {
     CB_REQUIRE(a->top_vals && a->cum && a->length && a->anc_in && a->best_key && a->best_len,
@@ -37,6 +40,9 @@ extern "C" int case_beam_select(const case_select_args_t* a, case_stream_t strea
     CB_REQUIRE(a->W == 1, "case_beam_select: greedy modes need W == 1");
     CB_REQUIRE(a->mode != CASE_MODE_PROTO_GREEDY || a->ended, "case_beam_select: proto-greedy needs ended[]");
   }
-  launch_k(beam_select_kernel, a->B, 32, 0, (cudaStream_t)stream, *a);
+  if (a->out_attr != nullptr)
+    launch_k(beam_select_kernel<true>, a->B, 32, 0, (cudaStream_t)stream, *a);
+  else
+    launch_k(beam_select_kernel<false>, a->B, 32, 0, (cudaStream_t)stream, *a);
   return check_launch("case_beam_select");
 }

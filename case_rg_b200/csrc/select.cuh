@@ -14,9 +14,34 @@ static inline int check_nbest(int nbest, int W, int mode) {
   return 0;
 }
 
+// Attribution (case_select_args_t.attr_*) is all three pointers or none; the caller picks the instance of the select
+static inline int check_attr_select(const case_select_args_t& a) {
+  const int n = (a.attr_cand != nullptr) + (a.attr_hist != nullptr) + (a.out_attr != nullptr);
+  CB_REQUIRE(n == 0 || n == 3, "attribution needs attr_cand, attr_hist and out_attr (or none of them)");
+  return 0;
+}
+
+__device__ __forceinline__ case_attr_t attr_zero() {
+  case_attr_t z;
+  z.part[0] = z.part[1] = z.part[2] = 0.f;
+  z.source = -1;
+  return z;
+}
+
+// a record written by another CTA of the same launch (fused form): L2 load, as top_vals
+__device__ __forceinline__ case_attr_t attr_ldcg(const case_attr_t* p) {
+  const float4 v = __ldcg(reinterpret_cast<const float4*>(p));
+  case_attr_t r;
+  r.part[0] = v.x; r.part[1] = v.y; r.part[2] = v.z; r.source = __float_as_int(v.w);
+  return r;
+}
+
 // One warp runs the bookkeeping of query b (all 32 lanes must call).  top_vals / top_idx may have been
 // written by other CTAs of the same launch (fused form: the last CTA of the query's W rows calls this
-// after a fence + atomic), hence the L2 (.cg) loads.
+// after a fence + atomic), hence the L2 (.cg) loads.  ATTR: the attribution records (case_select_args_t.attr_*) travel
+// with the tokens - candidate c of the query is attr_cand[r0 * W + c], kept children write attr_hist next to tok, the
+// finished rows copy it along the anc path like out_tokens.
+template <bool ATTR = false>
 __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, int b, int lane) {
   const int W = a.W, t = a.t, TL = a.Tmax + 1;
   const int r0 = b * W;
@@ -28,14 +53,17 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
   if (a.mode != CASE_MODE_BEAM) {   // W == 1
     if (lane == 0) {
       int tk = __ldcg(a.top_idx + r0);
+      bool padded = false;
       if (a.mode == CASE_MODE_PROTO_GREEDY) {
         const int was_ended = a.ended[b];
         const int this_end = tk == a.EOS;
         if (t == 0) { if (this_end) tk = a.UNK; }          // Generations.py:99-100
-        else if (was_ended) tk = a.PAD;                    // Generations.py:101-102
+        else if (was_ended) { tk = a.PAD; padded = true; } // Generations.py:101-102
         a.ended[b] = was_ended | this_end;
       }
       a.out_tokens[(size_t)b * a.Tmax + t] = tk;
+      // the record of the id the distribution chose (an EOS rewritten to UNK keeps it); PAD after the end: zero record
+      if constexpr (ATTR) a.out_attr[(size_t)b * a.Tmax + t] = padded ? attr_zero() : attr_ldcg(a.attr_cand + r0);
       a.tok[(size_t)r0 * TL + t + 1] = feed(tk);
       if (ext) tok_o[(size_t)r0 * TL + t + 1] = tk;
       a.parent[r0] = r0;
@@ -120,6 +148,7 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
       a.length[rn] = clen[c];
       a.live[rn] = 1;
       a.parent[rn] = pr;
+      if constexpr (ATTR) a.attr_hist[(size_t)rn * TL + t + 1] = attr_ldcg(a.attr_cand + (size_t)r0 * W + c);
     }
   }
   for (int w = s_nlive + lane; w < W; w += 32) {     // dead slots: harmless, in-range contents
@@ -128,6 +157,7 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
     a.parent[rn] = rn;
     a.tok[(size_t)rn * TL + t + 1] = a.PAD;
     if (ext) tok_o[(size_t)rn * TL + t + 1] = a.PAD;
+    if constexpr (ATTR) a.attr_hist[(size_t)rn * TL + t + 1] = attr_zero();
     for (int j = 0; j <= t; ++j) a.anc_out[(size_t)rn * TL + j] = rn;
   }
   // record the inserted finished sequences in insertion order: BOS dropped, EOS kept (:188).  Lane j owns column j of
@@ -146,6 +176,18 @@ __device__ __forceinline__ void beam_select_query(const case_select_args_t& a, i
         v = ctok[c];
       }
       out[(size_t)pos * a.Tmax + j] = v;
+      if constexpr (ATTR) {                              // the records ride the same path
+        case_attr_t* oa = a.out_attr + (size_t)b * nb * a.Tmax;
+        for (int i = nb - 1; i > pos; --i) oa[(size_t)i * a.Tmax + j] = oa[(size_t)(i - 1) * a.Tmax + j];
+        case_attr_t e = attr_zero();
+        if (j < t) {
+          const int src = (j + 1 == t) ? pr : a.anc_in[(size_t)pr * TL + j + 1];
+          e = a.attr_hist[(size_t)src * TL + j + 1];
+        } else if (j == t) {
+          e = attr_ldcg(a.attr_cand + (size_t)r0 * W + c);
+        }
+        oa[(size_t)pos * a.Tmax + j] = e;
+      }
     }
   }
 }

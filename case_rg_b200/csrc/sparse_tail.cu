@@ -138,6 +138,9 @@ __global__ __launch_bounds__(ST) void vocab_base_kernel(const float* __restrict_
 __device__ __forceinline__ uint32_t sp_hash(int id, int shift) { return ((uint32_t)id * 2654435761u) >> shift; }
 __device__ __forceinline__ uint32_t sp_step(int id) { return (((uint32_t)id * 40503u) >> 4) | 1u; }
 
+// ATTR (case_tail_args_t.attr != NULL): after the top-k, an attribution pass writes the record of every winner (see
+// below); the fused select then carries the records with the tokens
+template <bool ATTR>
 __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t a, const float* __restrict__ base_ms,
                                                          const float* __restrict__ base_e,
                                                          const int32_t* __restrict__ base_i, int k2, int nslots,
@@ -504,6 +507,80 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
     a.top_idx[(size_t)r * K + lane] = oi;
   }
   stamp();
+  if constexpr (ATTR) {
+    // ---- attribution of the K winners: the source positions are walked again (the same map / score / prior loads as
+    // the hash pass, which just read them, so they come from L2) and a position whose id is a winner adds its
+    // contribution to the (winner, memory) accumulator - in the fixed point and with the split-word atomics of the hash
+    // table, so in hash mode the two copy parts add up, as integers, to exactly the mass the ranking used - and offers
+    // (float bits of the contribution, ~position) to one 64-bit maximum: contributions are positive, so the bit order
+    // is the value order, and ties go to the lowest position.  Independent of the copy plan.
+    __shared__ int s_aid[CASE_MAX_W];
+    __shared__ uint32_t s_alo[CASE_MAX_W][2], s_ahi[CASE_MAX_W][2];
+    __shared__ unsigned long long s_asrc[CASE_MAX_W];
+    if (tid < CASE_MAX_W) {                                // warp 0: lane k < K holds winner k
+      s_aid[tid] = tid < K ? oi : -1;
+      s_alo[tid][0] = s_alo[tid][1] = s_ahi[tid][0] = s_ahi[tid][1] = 0u;
+      s_asrc[tid] = 0ull;
+    }
+    __syncthreads();
+    const int S0n = a.S[0], S1n = a.nmem > 1 ? a.S[1] : 0, Stot = S0n + S1n;
+    const float* at0 = a.attn_un[0] + (size_t)r * S0n;
+    const float* at1 = a.nmem > 1 ? a.attn_un[1] + (size_t)r * S1n : nullptr;
+    const float* pr0 = a.prior[0] ? a.prior[0] + (size_t)b * S0n : nullptr;
+    const float* pr1 = (a.nmem > 1 && a.prior[1]) ? a.prior[1] + (size_t)b * S1n : nullptr;
+    const int32_t* mp0 = a.map + (size_t)b * a.map_ld + a.map_off[0];
+    const int32_t* mp1 = a.map + (size_t)b * a.map_ld + a.map_off[1];
+    constexpr int HU = 4;                                  // positions per thread per round (loads from L2)
+    for (int s0 = tid; s0 < Stot; s0 += HU * TS) {
+      int id[HU];
+      float ev[HU], pv[HU];
+#pragma unroll
+      for (int u = 0; u < HU; ++u) {
+        const int sidx = s0 + u * TS;
+        const bool in = sidx < Stot, m1 = sidx >= S0n;
+        const int sl = m1 ? sidx - S0n : sidx;
+        const float* pr = m1 ? pr1 : pr0;
+        id[u] = in ? __ldg((m1 ? mp1 : mp0) + sl) : -1;
+        ev[u] = in ? (m1 ? at1 : at0)[sl] : -INFINITY;
+        pv[u] = (in && pr) ? __ldg(pr + sl) : 1.f;
+      }
+#pragma unroll
+      for (int u = 0; u < HU; ++u) {
+        if (ev[u] == -INFINITY || (unsigned)id[u] >= (unsigned)Vx) continue;
+        int k = -1;
+        for (int j = 0; j < K; ++j) k = id[u] == s_aid[j] ? j : k;
+        if (k < 0) continue;
+        const int sidx = s0 + u * TS;
+        const bool m1 = sidx >= S0n;
+        const float cw = (m1 ? F[1] : F[0]) * pv[u] * fexp(ev[u] - (m1 ? M[1] : M[0]));   // as in the hash pass
+        const unsigned long long q = __float2ull_rn(fminf(cw, 32768.f) * 281474976710656.f);
+        if (q == 0ull) continue;                           // below the fixed point's resolution: no contribution
+        const uint32_t lo = (uint32_t)q;
+        const uint32_t prev = atomicAdd(&s_alo[k][m1], lo);
+        const uint32_t hi = (uint32_t)(q >> 32) + ((uint32_t)(prev + lo) < prev ? 1u : 0u);
+        if (hi) atomicAdd(&s_ahi[k][m1], hi);
+        atomicMax(&s_asrc[k], ((unsigned long long)__float_as_uint(cw) << 32) | (0xFFFFFFFFu - (uint32_t)sidx));
+      }
+    }
+    __syncthreads();
+    if (tid < K) {
+      const int y = s_aid[tid];
+      case_attr_t rec;
+      rec.part[0] = rec.part[1] = rec.part[2] = 0.f;
+      rec.source = -1;
+      if ((unsigned)y < (unsigned)Vx) {
+        // generation part: the expression the value was built from
+        const float e = ((a.mask_col0 && y == 0) || y >= V) ? 0.f : sp_exp(x[y] - mm);
+        rec.part[0] = scl * e;
+#pragma unroll
+        for (int i = 0; i < 2; ++i)
+          rec.part[1 + i] = __ull2float_rn(((unsigned long long)s_ahi[tid][i] << 32) | s_alo[tid][i]) * 3.552713678800501e-15f;
+        const unsigned long long key = s_asrc[tid];
+        if (key) rec.source = (int)(0xFFFFFFFFu - (uint32_t)key);
+      }
+      a.attr[(size_t)r * K + tid] = rec;
+    }
+  }
   // ---- fused search bookkeeping: the last CTA of a query's W rows runs Generations.beam / greedy for it
   if (do_select) {
     __shared__ int s_last;
@@ -517,7 +594,7 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
       if (s_last) qcount[b] = 0;                          // ready for the next step
     }
     __syncthreads();
-    if (s_last && warp == 0) beam_select_query(sel, b, lane);
+    if (s_last && warp == 0) beam_select_query<ATTR>(sel, b, lane);
   }
 }
 
@@ -567,17 +644,23 @@ extern "C" int case_sparse_tail(const case_tail_args_t* a, const float* base_ms,
   const size_t smem = plan ? (size_t)((total + 3) / 4 * 4) * 8 : (size_t)nslots * 12;
   if (plan) nslots = (total + 3) / 4 * 4;
   if (sel) {
-    const int rc = check_nbest(sel->nbest, sel->W, sel->mode);
+    int rc = check_nbest(sel->nbest, sel->W, sel->mode);
     if (rc) return rc;
+    rc = check_attr_select(*sel);
+    if (rc) return rc;
+    CB_REQUIRE((sel->out_attr != nullptr) == (a->attr != nullptr) && (sel->attr_cand == nullptr || sel->attr_cand == a->attr),
+               "case_sparse_tail: a fused select with attribution needs attr_cand == the tail's attr (both on or both off)");
   }
+  const bool attr = a->attr != nullptr;
   cudaStream_t st = (cudaStream_t)stream;
-  ensure_smem<sparse_tail_kernel>(16384 * 12);
+  if (attr) ensure_smem<sparse_tail_kernel<true>>(16384 * 12);
+  else ensure_smem<sparse_tail_kernel<false>>(16384 * 12);
   CB_REQUIRE(sel == nullptr || (qcount != nullptr && sel->B * sel->W == a->R && sel->W == a->W && a->K == a->W),
              "case_sparse_tail: fused select needs qcount and matching B / W (k = W)");
   case_select_args_t sv;
   memset(&sv, 0, sizeof(sv));
   if (sel) sv = *sel;
-  launch_k(sparse_tail_kernel, a->R, TS, smem, st, *a, base_ms, base_e, base_i, k2, nslots, g_sp_dbg, sv, sel ? 1 : 0,
-           qcount);
+  launch_k(attr ? sparse_tail_kernel<true> : sparse_tail_kernel<false>, a->R, TS, smem, st, *a, base_ms, base_e, base_i, k2,
+           nslots, g_sp_dbg, sv, sel ? 1 : 0, qcount);
   return check_launch("case_sparse_tail");
 }

@@ -123,18 +123,31 @@ static case_select_args_t select_args(int mode, int B, int W, int t, int max_len
   return s;
 }
 
-static int select_step(int mode, int B, int W, int t, int max_len, int Tmax, int BOS, int EOS, int UNK, int PAD,
-                       const float* top_vals, const int32_t* top_idx, int32_t* live, double* cum, int32_t* length,
-                       int32_t* tok, int32_t* const anc[2], int32_t* parent, int32_t* ended, double* best_key,
-                       int32_t* best_len, int32_t* out_tokens, int32_t* n_live, int nbest, cudaStream_t st) {
-  case_select_args_t s;
-  memset(&s, 0, sizeof(s));
-  s.mode = mode; s.B = B; s.W = W; s.t = t; s.max_len = max_len; s.Tmax = Tmax;
-  s.BOS = BOS; s.EOS = EOS; s.UNK = UNK; s.PAD = PAD;
-  s.top_vals = top_vals; s.top_idx = top_idx; s.live = live; s.cum = cum; s.length = length; s.tok = tok;
-  s.anc_in = anc[t & 1]; s.anc_out = anc[(t + 1) & 1]; s.parent = parent; s.ended = ended;
-  s.best_key = best_key; s.best_len = best_len; s.out_tokens = out_tokens; s.n_live = n_live; s.nbest = nbest;
-  return case_beam_select(&s, st);
+// Attribution records of a step (the attr_* fields of the step blocks): all three or none, and only where the step takes
+// the sparse tail - the only tail with an attribution pass.  Checked before the first launch of the step.
+static int check_step_attr(const case_attr_t* cand, const case_attr_t* hist, const case_attr_t* out, bool sparse,
+                           const char* what) {
+  const int n = (cand != nullptr) + (hist != nullptr) + (out != nullptr);
+  if (n == 0) return 0;
+  if (n != 3) {
+    char msg[160];
+    snprintf(msg, sizeof(msg), "%s: attribution needs attr_cand, attr_hist and out_attr (or none of them)", what);
+    set_error(msg);
+    return CASE_EINVAL;
+  }
+  if (!sparse) {
+    char msg[256];
+    snprintf(msg, sizeof(msg), "%s: attribution needs the sparse tail (not with CASE_OPT_DENSE_TAIL / UNFUSED_TAIL, "
+             "materialize_only, missing base_* buffers, V < 2W or too many source positions)", what);
+    set_error(msg);
+    return CASE_EINVAL;
+  }
+  return 0;
+}
+
+static void set_select_attr(case_select_args_t& s, case_attr_t* cand, case_attr_t* hist, case_attr_t* out) {
+  if (out == nullptr) return;
+  s.attr_cand = cand; s.attr_hist = hist; s.out_attr = out;
 }
 
 extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t stream) {
@@ -163,6 +176,8 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
   const int k2 = 2 * W;
   const bool sparse = use_tail == 2 && !a->materialize_only && a->base_ms && a->base_e && a->base_i && a->V >= k2 &&
                       a->S[0] + a->S[1] <= case_sparse_tail_max_sources();
+  TRY(check_step_attr(a->attr_cand, a->attr_hist, a->out_attr, sparse, "case_decode_step"));
+  const bool attr = a->out_attr != nullptr;
   // gate form of the additive attentions: the contexts only feed the mixture gate, so 3 gate-projected numbers
   // per key replace the value rows (needs the sparse tail, which merges gate partials instead of contexts)
   const bool gate = !(opt & CASE_OPT_NO_GATE) && sparse && dt == CASE_BF16 && a->Gv[0] != nullptr && a->Gv[1] != nullptr;
@@ -357,12 +372,14 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
       ta.cp_n = a->cp_n; ta.cp_uid = a->cp_uid; ta.cp_first = a->cp_first; ta.cp_start = a->cp_start; ta.cp_perm = a->cp_perm;
       ta.cp_ld = a->cp_ld;
     }
+    if (attr) ta.attr = a->attr_cand;
     if (sparse) {
       const bool fuse_sel = a->qcount != nullptr && !(opt & CASE_OPT_NO_FUSED_SELECT);
       case_select_args_t sel = select_args(a->mode, B, W, t, a->max_len, a->Tmax, a->BOS, a->EOS, a->UNK, a->PAD,
                                            a->top_vals, a->top_idx, a->live, a->cum, a->length, a->tok, a->anc, a->parent,
                                            a->ended, a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
       if (n_oov) { sel.V_in = a->V; sel.tok_ext = a->tok_ext; }
+      set_select_attr(sel, a->attr_cand, a->attr_hist, a->out_attr);
       TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2, fuse_sel ? &sel : nullptr, a->qcount, st));
       if (fuse_sel) return 0;
     } else {
@@ -387,6 +404,7 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
                                          a->top_idx, a->live, a->cum, a->length, a->tok, a->anc, a->parent, a->ended,
                                          a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
     if (n_oov) { sel.V_in = a->V; sel.tok_ext = a->tok_ext; }
+    set_select_attr(sel, a->attr_cand, a->attr_hist, a->out_attr);
     return case_beam_select(&sel, st);
   }
 }
@@ -413,6 +431,12 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
   const int opt = a->opt;
   OptScope scope(opt);
   const int use_tail = (opt & CASE_OPT_UNFUSED_TAIL) ? 0 : 1;
+  // search path: the sparse tail of the CaSE step (base statistics of the logits + the copy mass hashed by vocabulary id,
+  // accumulated in fixed point: the top-k never needs the [R, V] mixture and is reproducible run to run)
+  const int k2 = 2 * W <= 2 * CASE_MAX_W ? 2 * W : 2 * CASE_MAX_W;
+  const bool sparse = use_tail && !(opt & CASE_OPT_DENSE_TAIL) && !a->materialize_only && a->base_ms && a->base_e && a->base_i &&
+                      a->V >= k2 && a->Lb <= case_sparse_tail_max_sources();
+  TRY(check_step_attr(a->attr_cand, a->attr_hist, a->out_attr, sparse, "gttp_decode_step"));
 
   TRY(case_embed_rows(a->E, nullptr, a->tok, TL, t, 1.0f, a->emb, R, st));
   // two additive attentions with the previous GRU state as query (GTTP/Model.py:117-122)
@@ -478,11 +502,6 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
   }
   TRY(case_vocab_gemm(a->feat, a->Wv, a->bv, a->logits, R, a->V, a->ldv, dt, a->vocab_impl, a->vocab_ws, st));
   TRY(case_gttp_gates(a->feat, a->wc, a->bc, a->gates, a->fac, CASE_MAX_SPLIT, ns[1], R, st));
-  // search path: the sparse tail of the CaSE step (base statistics of the logits + the copy mass hashed by vocabulary id,
-  // accumulated in fixed point: the top-k never needs the [R, V] mixture and is reproducible run to run)
-  const int k2 = 2 * W <= 2 * CASE_MAX_W ? 2 * W : 2 * CASE_MAX_W;
-  const bool sparse = use_tail && !(opt & CASE_OPT_DENSE_TAIL) && !a->materialize_only && a->base_ms && a->base_e && a->base_i &&
-                      a->V >= k2 && a->Lb <= case_sparse_tail_max_sources();
   if (sparse) {
     TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 1, k2, a->base_ms, a->base_e, a->base_i, st));
     case_tail_args_t ta;
@@ -492,6 +511,7 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
     ta.logits = a->logits; ta.gates = a->gates; ta.fac = a->fac; ta.map = a->map;
     ta.S[0] = a->Lb; ta.attn_un[0] = a->attn_un[1];
     ta.top_vals = a->top_vals; ta.top_idx = a->top_idx;
+    ta.attr = a->attr_cand;
     TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2, nullptr, nullptr, st));
   } else if (use_tail && a->V <= case_row_tail_max_vocab()) {
     case_tail_args_t ta;
@@ -510,9 +530,11 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
     if (a->materialize_only) return 0;
     TRY(case_topk_rows(a->dist, a->ldv, R, a->V, W, a->top_vals, a->top_idx, st));
   }
-  return select_step(a->mode, B, W, t, a->max_len, a->Tmax, a->BOS, a->EOS, a->UNK, a->PAD, a->top_vals, a->top_idx,
-                     a->live, a->cum, a->length, a->tok, a->anc, a->parent, a->ended, a->best_key, a->best_len,
-                     a->out_tokens, a->n_live, a->nbest, st);
+  case_select_args_t sel = select_args(a->mode, B, W, t, a->max_len, a->Tmax, a->BOS, a->EOS, a->UNK, a->PAD, a->top_vals,
+                                       a->top_idx, a->live, a->cum, a->length, a->tok, a->anc, a->parent, a->ended,
+                                       a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
+  set_select_attr(sel, a->attr_cand, a->attr_hist, a->out_attr);
+  return case_beam_select(&sel, st);
 }
 
 /* layout self-check for FFI bindings: sizeof of each argument struct, by index */

@@ -321,11 +321,55 @@ def nbest_from(out_tokens, best_len, best_key) -> NBest:
                  best_key.reshape(B, n).clone())
 
 
+class Attributed(NamedTuple):
+    """Answers with the attribution record of every token: where its probability came from in the mixture of its parent
+    prefix (CaSE/Model.py:38-48, GTTP/Model.py:25-43).  ``answer``: the search's own result (the ``beam_nbest`` NBest,
+    or the LongTensor of ``greedy`` / ``beam``).  ``parts`` fp32 [..., L, P]: the split of the chosen token's probability
+    p(y) - the ``p`` whose -log(p + 1e-10) entered the cost - into P parts that sum to it: CaSE (P = 3) generation, copy
+    from the query, copy from the passages; GTTP (P = 2) generation, copy from the background.  ``source`` int64
+    [..., L]: the source position with the largest single copy contribution to the token (an index of ``source_map`` /
+    ``background_map``, ties to the lowest position; see ``results.source_location``), -1 for pure generation.
+    Positions past an answer's end (and greedy PAD positions) have zero parts and source -1."""
+    answer: object
+    parts: torch.Tensor
+    source: torch.Tensor
+
+
+def attributed_from(out_tokens, best_len, best_key, out_attr, P, mode, max_len, nbest) -> Attributed:
+    """Search-state buffers (out_tokens [B, (n,) T], best_len / best_key [B, (n)], out_attr [B, (n,) T, 4] fp32 records)
+    -> Attributed on their device.  nbest: the answer is the NBest list and the records are [B, n, L, ...]; otherwise the
+    answer is entry 0's token rows ([B, max_len] greedy; beam trimmed to the longest answer) and the records [B, L, ...]."""
+    B = best_len.size(0)
+    rec = out_attr.reshape(B, -1, out_attr.size(-2), 4)[:, :, :max_len]
+    if mode == L.MODE_BEAM:
+        rec = rec[:, :, :max(int(best_len.max()), 1)]         # merge1D, like the token rows
+    parts = rec[..., :P].clone()
+    source = rec[..., 3].contiguous().view(torch.int32).to(torch.int64)
+    if nbest:
+        return Attributed(nbest_from(out_tokens, best_len, best_key), parts, source)
+    toks = out_tokens.reshape(B, -1, out_tokens.size(-1))[:, 0, :rec.size(2)].to(torch.int64)
+    return Attributed(toks, parts[:, 0], source[:, 0])
+
+
+def check_attribution(opt: int, V: int, W: int, nsources: int) -> None:
+    """Attribution records come from the sparse tail only: ValueError for a request the step would refuse."""
+    if opt & (L.OPT_DENSE_TAIL | L.OPT_UNFUSED_TAIL):
+        raise ValueError('attribution needs the sparse tail: not with OPT_DENSE_TAIL / OPT_UNFUSED_TAIL')
+    if V < 2 * W:
+        raise ValueError(f'attribution needs the sparse tail, which needs V >= 2 * width (V = {V}, width = {W})')
+    if nsources > L.load().case_sparse_tail_max_sources():
+        raise ValueError(f'attribution needs the sparse tail: {nsources} source positions exceed its '
+                         f'{L.load().case_sparse_tail_max_sources()}')
+
+
 class _SearchState:
     """Buffers shared by both engines for the on-device greedy / beam bookkeeping.  nbest > 1: the beam search keeps
-    the nbest best finished hypotheses of every query (best_key / best_len [B, nbest], out_tokens [B, nbest, Tmax])."""
+    the nbest best finished hypotheses of every query (best_key / best_len [B, nbest], out_tokens [B, nbest, Tmax]).
+    attribution: the records of the search (case_attr_t as fp32 [..., 4], the source bits in the last lane) - of the
+    top-k candidates attr_cand [R, W], of every (physical row, position) attr_hist [R, Tmax + 1], and of the returned
+    tokens out_attr (the layout of out_tokens)."""
 
-    def __init__(self, dev, B, W, Tmax, ext=False, nbest=1):
+    def __init__(self, dev, B, W, Tmax, ext=False, nbest=1, attribution=False):
         if not 1 <= nbest <= W:
             raise ValueError(f'nbest must be 1..{W} (the beam width), got {nbest}')
         R, TL = B * W, Tmax + 1
@@ -344,6 +388,12 @@ class _SearchState:
         self.best_len = torch.zeros(B, *nb, **i32)
         self.out_tokens = torch.zeros(B, *nb, Tmax, **i32)
         self.n_live = torch.zeros(B, **i32)
+        self.attribution = bool(attribution)
+        if self.attribution:
+            f32 = dict(dtype=torch.float32, device=dev)
+            self.attr_cand = torch.zeros(R, W, 4, **f32)
+            self.attr_hist = torch.zeros(R, TL, 4, **f32)
+            self.out_attr = torch.zeros(B, *nb, Tmax, 4, **f32)
         self.B, self.W, self.R, self.Tmax, self.nbest = B, W, R, Tmax, nbest
         self._arange = torch.arange(R, **i32)
         self._slot0 = (self._arange % W == 0).to(torch.int32)
@@ -364,12 +414,19 @@ class _SearchState:
         self.best_len.zero_()
         self.out_tokens.zero_()
         self.n_live.zero_()
+        if self.attribution:                    # zero records: parts 0, source -1
+            for r in (self.attr_hist, self.out_attr):
+                r.zero_()
+                r[..., 3].view(torch.int32).fill_(-1)
 
     def bind(self, a):
         a.anc[0], a.anc[1] = self.anc[0].data_ptr(), self.anc[1].data_ptr()
         for n in ('tok', 'live', 'cum', 'length', 'parent', 'ended', 'best_key', 'best_len', 'out_tokens', 'n_live'):
             setattr(a, n, getattr(self, n).data_ptr())
         a.nbest = self.nbest
+        if self.attribution:
+            a.attr_cand, a.attr_hist, a.out_attr = (self.attr_cand.data_ptr(), self.attr_hist.data_ptr(),
+                                                    self.out_attr.data_ptr())
 
 
 class _EngineBase:
@@ -426,19 +483,31 @@ class _EngineBase:
         st = self.state
         return nbest_from(st.out_tokens, st.best_len, st.best_key)
 
+    def _finish_attribution(self, max_len: int, mode: int, nbest: bool = False) -> Attributed:
+        """The answers and attribution records of the last decode of an engine built with attribution=True (see
+        Attributed); nbest: the answer is the NBest list and the records carry its n axis."""
+        st = self.state
+        if not st.attribution:
+            raise ValueError('this engine was built without attribution=True')
+        return attributed_from(st.out_tokens, st.best_len, st.best_key, st.out_attr, self.nparts, mode, max_len, nbest)
+
 
 class CaseDecodeEngine(_EngineBase):
     """All buffers + the step argument block for one CaSE problem shape."""
 
     def __init__(self, weights: CaseWeights, B: int, W: int, S0: int, S1: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0, n_oov: int = 0, nbest: int = 1):
+                 opt: int = 0, n_oov: int = 0, nbest: int = 1, attribution: bool = False):
         """n_oov > 0: extended vocabulary - ``source_map`` entries in [V, V + n_oov) are per-query dynamic (OOV) words,
         the mixture and its top-k range over V + n_oov ids (pointer-generator extension; an OOV id is fed back as UNK).
-        nbest (1..W): a beam decode keeps the nbest best finished hypotheses per query (read with ``_finish_nbest``)."""
+        nbest (1..W): a beam decode keeps the nbest best finished hypotheses per query (read with ``_finish_nbest``).
+        attribution: every decode also records where each answer token came from (read with ``_finish_attribution``)."""
         self.opt, self.n_oov = int(opt), int(n_oov)
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
+        if attribution:
+            check_attribution(self.opt, weights.V, W, S0 + S1)
+        self.nparts = 3
         if not (1 <= Tmax <= L.MAX_T):
             raise ValueError(f'max_target_length must be 1..{L.MAX_T}')
         self.w = weights
@@ -480,7 +549,7 @@ class CaseDecodeEngine(_EngineBase):
         # state
         self.kcache = [torch.zeros(R, Tmax, H, dtype=td, device=dev) for _ in range(8)]
         self.vcache = [torch.zeros(R, Tmax, H, dtype=td, device=dev) for _ in range(8)]
-        self.state = _SearchState(dev, B, W, Tmax, ext=self.n_oov > 0, nbest=nbest)
+        self.state = _SearchState(dev, B, W, Tmax, ext=self.n_oov > 0, nbest=nbest, attribution=attribution)
         # scratch
         # second memory: only valid keys are packed (case_cross_attn_part); CASE_NO_COMPACT=1 keeps the masked form (A/B)
         self.compact = weights.cdtype == L.BF16 and os.environ.get('CASE_NO_COMPACT', '0') != '1'
@@ -536,7 +605,7 @@ class CaseDecodeEngine(_EngineBase):
         self._fill_args()
 
     def _fill_args(self):
-        a = self.args = L.StepArgs()
+        a = self.args = L.StepAttrArgs()
         w = self.w
         a.opt, a.fork = self.opt, self._fork.h
         if self.n_oov:
@@ -750,9 +819,12 @@ class GttpWeights:
 class GttpDecodeEngine(_EngineBase):
     def __init__(self, weights: GttpWeights, B: int, W: int, Lc: int, Lb: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0, nbest: int = 1):
+                 opt: int = 0, nbest: int = 1, attribution: bool = False):
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
+        if attribution:
+            check_attribution(int(opt), weights.V, W, Lb)
+        self.nparts = 2
         self.w = weights
         self.device = dev = weights.device
         self.B, self.W, self.R, self.Lc, self.Lb, self.Tmax, self.V = B, W, B * W, Lc, Lb, Tmax, weights.V
@@ -773,7 +845,7 @@ class GttpDecodeEngine(_EngineBase):
         self.mask = [torch.zeros(B, s, dtype=torch.uint8, device=dev) for s in (Lc, Lb)]
         self.map = torch.zeros(B, Lb, dtype=torch.int32, device=dev)
         self.gstate = [z(R, H), z(R, H)]
-        self.state = _SearchState(dev, B, W, Tmax, nbest=nbest)
+        self.state = _SearchState(dev, B, W, Tmax, nbest=nbest, attribution=attribution)
         self.emb, self.qa = z(R, H), z(R, H)
         self.attn_un = [z(R, Lc), z(R, Lb)]
         self.stats = [z(R, n, 4) for n in self.ns]
@@ -791,7 +863,7 @@ class GttpDecodeEngine(_EngineBase):
         self._graphs = {}
         self._step_fn = L.load().gttp_decode_step
         self._step_name = 'gttp_decode_step'
-        a = self.args = L.GttpStepArgs()
+        a = self.args = L.GttpStepAttrArgs()
         w = weights
         a.B, a.W, a.R, a.V, a.ldv, a.dtype = B, W, R, V, self.ldv, w.cdtype
         a.opt = int(opt)

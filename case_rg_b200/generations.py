@@ -9,6 +9,8 @@ zero-padded to the longest answer - ``merge1D``, common/Utils.py:366-377).
 
 ``beam_nbest`` returns more than the reference's single answer: the n best finished hypotheses of every query with
 their costs, the sorted ``results[q]`` list that Generations.beam builds and reads element 0 of (Generations.py:183-185).
+``beam_attributed`` / ``greedy_attributed`` also report where every answer token came from: the split of its
+probability into generation and copy from each memory, and the source position it was most copied from.
 
 ``FastCaSE`` gives the unchanged CaSE decoder the protocol the reference never implemented for it
 (SURVEY.md §8c adapter); ``FastGTTP`` replaces ``GTTP.decode/generate/to_word`` + the search
@@ -20,7 +22,8 @@ from typing import Dict, Optional
 import torch
 
 from . import _lib as L
-from .engine import CaseDecodeEngine, CaseWeights, GttpDecodeEngine, GttpWeights, NBest, nbest_from
+from .engine import (Attributed, CaseDecodeEngine, CaseWeights, GttpDecodeEngine, GttpWeights, NBest, attributed_from,
+                     nbest_from)
 
 PAD_WORD, BOS_WORD, UNK_WORD, EOS_WORD = '[PAD]', '[unused0]', '[UNK]', '[unused1]'
 
@@ -64,23 +67,51 @@ def beam_nbest(model, data, vocab2id=None, max_len=20, width=5, n=None, encode_o
     return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states, nbest=n)
 
 
-def beam_batches(model, batches, vocab2id=None, max_len=20, width=5, n_best=None):
+def beam_attributed(model, data, vocab2id=None, max_len=20, width=5, n=None, encode_outputs=None,
+                    init_decoder_states=None):
+    """``beam_nbest`` with the attribution record of every answer token: ``Attributed(answer, parts, source)`` on the
+    model's device, ``answer`` the NBest of ``beam_nbest`` (the same search, bit for bit), ``parts`` fp32 [B, n, L, P] and
+    ``source`` int64 [B, n, L], trimmed like the tokens (see engine.Attributed).  n defaults to the width."""
+    _check_vocab(vocab2id)
+    n = _nbest_count(n, width)
+    return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states, nbest=n,
+                             attribution=True)
+
+
+def greedy_attributed(model, data, vocab2id=None, max_len=20, encode_outputs=None, init_decoder_states=None):
+    """``greedy`` with the attribution record of every answer token: ``Attributed(answer, parts, source)``, ``answer`` the
+    LongTensor [B, max_len] of ``greedy``, ``parts`` fp32 [B, max_len, P], ``source`` int64 [B, max_len].  At t = 0 an
+    EOS rewritten to UNK keeps the record of the EOS the distribution chose; PAD positions after the end have zero parts
+    and source -1."""
+    _check_vocab(vocab2id)
+    return model.fast_search(data, max_len, 1, L.MODE_PROTO_GREEDY, encode_outputs, init_decoder_states,
+                             attribution=True)
+
+
+def beam_batches(model, batches, vocab2id=None, max_len=20, width=5, n_best=None, attribution=False):
     """``beam`` over an iterable of HOST batches, the way the predict loop feeds a model one batch after
     another (common/CumulativeTrainer.py:141-156): yields the answers of every batch, in order, as host
     LongTensors.  The host-to-device copy of batch i+1 runs on a copy stream while batch i is decoding
     (double-buffered staging, pinned host tensors copy asynchronously), so the PCIe time of the encoder
     outputs (175 MB per batch at the BASELINE shape) is hidden behind the decode.  n_best: yields the ``beam_nbest``
-    lists of every batch instead (NBest of host tensors)."""
+    lists of every batch instead (NBest of host tensors).  attribution: yields what ``beam_attributed(..., n=n_best)``
+    returns for every batch (host Attributed; n_best None = the width)."""
     _check_vocab(vocab2id)
-    if n_best is not None:
+    if n_best is not None or attribution:
         n_best = _nbest_count(n_best, width)
-    return model.search_batches(batches, max_len, width, L.MODE_BEAM, n_best)
+    return model.search_batches(batches, max_len, width, L.MODE_BEAM, n_best, attribution)
 
 
-def greedy_batches(model, batches, vocab2id=None, max_len=20):
-    """``greedy`` over an iterable of host batches with the copy of the next batch overlapped (see beam_batches)."""
+def greedy_batches(model, batches, vocab2id=None, max_len=20, attribution=False):
+    """``greedy`` over an iterable of host batches with the copy of the next batch overlapped (see beam_batches).
+    attribution: yields what ``greedy_attributed`` returns for every batch (host Attributed)."""
     _check_vocab(vocab2id)
-    return model.search_batches(batches, max_len, 1, L.MODE_PROTO_GREEDY)
+    return model.search_batches(batches, max_len, 1, L.MODE_PROTO_GREEDY, None, attribution)
+
+
+def _to_host(att: Attributed) -> Attributed:
+    ans = NBest(*(x.cpu() for x in att.answer)) if isinstance(att.answer, NBest) else att.answer.cpu()
+    return Attributed(ans, att.parts.cpu(), att.source.cpu())
 
 
 class _FastModel:
@@ -109,9 +140,12 @@ class _FastModel:
         return to_sentence(batch_indices, self.id2vocab)
 
     # ---- streamed batches (beam_batches / greedy_batches)
-    def search_batches(self, batches, max_len, width, mode, n_best=None):
-        """Generator behind beam_batches / greedy_batches (n_best: beam mode, yields NBest per batch)."""
+    def search_batches(self, batches, max_len, width, mode, n_best=None, attribution=False):
+        """Generator behind beam_batches / greedy_batches (n_best: beam mode, yields NBest per batch; attribution: yields
+        Attributed per batch)."""
         dev = self.weights.device
+        if attribution:
+            self._check_attribution_opt()
         main = torch.cuda.current_stream(dev)
         # the copy stream and the two staging sets live as long as the model: allocating 2 x 175 MB on a
         # fresh stream per call costs tens of milliseconds of cudaMalloc
@@ -150,7 +184,7 @@ class _FastModel:
             # decoding is never prefilled: engine_for returns the SAME engine for equal shapes, and its decode is
             # ahead of this prefill on the main stream)
             main.wait_event(ready)
-            eng = self._prefill_staged(d, width, max_len, n_best or 1)
+            eng = self._prefill_staged(d, width, max_len, n_best or 1, attribution)
             prefilled[k] = torch.cuda.Event()
             prefilled[k].record(main)
             nxt = next(it, None)
@@ -164,24 +198,28 @@ class _FastModel:
                 # stream - the device never idles while the host reads answers
                 st = pending.state
                 snap = (st.out_tokens[..., :max_len].clone(), st.best_len.clone()) + \
-                    ((st.best_key.clone(),) if n_best else ())
+                    ((st.best_key.clone(),) if n_best or attribution else ()) + \
+                    ((st.out_attr[..., :max_len, :].clone(),) if attribution else ())
                 ev = torch.cuda.Event()
                 ev.record(main)
                 eng.launch(max_len, mode, use_graph=self.use_graph)
-                yield self._read_snapshot(snap, ev, mode)
+                yield self._read_snapshot(snap, ev, mode, (pending.nparts, max_len, n_best) if attribution else None)
             else:
                 eng.launch(max_len, mode, use_graph=self.use_graph)
             self.last_engine = pending = eng
             k ^= 1
         if pending is not None:
-            if n_best:
+            if attribution:
+                yield _to_host(pending._finish_attribution(max_len, mode, mode == L.MODE_BEAM))
+            elif n_best:
                 yield NBest(*(x.cpu() for x in pending._finish_nbest()))
             else:
                 yield pending._finish_tokens(max_len, mode).cpu()
 
-    def _read_snapshot(self, snap, ev, mode):
-        """Device snapshot (tokens [B, T] int32, best_len [B], or with best_key [B, n] the n-best buffers) -> host int64
-        tokens trimmed like _finish_tokens, or the host NBest."""
+    def _read_snapshot(self, snap, ev, mode, attr=None):
+        """Device snapshot (tokens [B, T] int32, best_len [B], or with best_key [B, n] the n-best buffers, with out_attr
+        the attribution records too) -> host int64 tokens trimmed like _finish_tokens, the host NBest, or with attr =
+        (parts, max_len, n_best) the host Attributed."""
         dev = self.weights.device
         if getattr(self, '_d2h_stream', None) is None:
             self._d2h_stream = torch.cuda.Stream(dev)
@@ -190,6 +228,9 @@ class _FastModel:
         with torch.cuda.stream(d2h):
             host = [x.to('cpu', non_blocking=True) for x in snap]
         d2h.synchronize()
+        if attr is not None:
+            P, max_len, n_best = attr
+            return attributed_from(*host, P, mode, max_len, mode == L.MODE_BEAM)
         if len(host) == 3:
             return nbest_from(*host)
         toks, blen = host
@@ -197,6 +238,19 @@ class _FastModel:
         if mode == L.MODE_BEAM:             # merge1D (Utils.py:366-377): pad to the longest answer of the batch
             out = out[:, :max(int(blen.max()), 1)]
         return out
+
+    def _check_attribution_opt(self):
+        """Attribution needs the sparse tail: refuse the option bits that switch it off before anything is built."""
+        if self.opt & (L.OPT_DENSE_TAIL | L.OPT_UNFUSED_TAIL):
+            raise ValueError('attribution needs the sparse tail: not with OPT_DENSE_TAIL / OPT_UNFUSED_TAIL')
+
+    def _finish(self, eng, max_len, mode, nbest, attribution):
+        """Answers of the decode just launched on ``eng``: tokens, the NBest list (nbest), or Attributed (attribution)."""
+        if attribution:
+            return eng._finish_attribution(max_len, mode, nbest is not None)
+        if nbest is None:
+            return eng._finish_tokens(max_len, mode)
+        return eng._finish_nbest()
 
 
 class FastCaSE(_FastModel):
@@ -223,10 +277,12 @@ class FastCaSE(_FastModel):
             from .producers import CaseProducers
             self.producers = CaseProducers(producers, device=self.weights.device)
 
-    def search_ids(self, data, max_len=None, width=None, mode='beam', n_best=None):
+    def search_ids(self, data, max_len=None, width=None, mode='beam', n_best=None, attribution=False):
         """CaSE.do_test from token ids (CaSE/Model.py:313-331): ``data`` = {'query' int [B,1,Lq], 'passage' int [B,NP,Lp],
         'source_map' int [B,S]} -> {'answer': LongTensor, 'rank': [B,NP]} like the reference's forward(data, 'test').
-        n_best (beam mode): also 'nbest', the ``beam_nbest`` list of the same search (its entry 0 is 'answer')."""
+        n_best (beam mode): also 'nbest', the ``beam_nbest`` list of the same search (its entry 0 is 'answer').
+        attribution (every mode): also 'attribution', the Attributed of the same search - its answer is the NBest with
+        n_best, else 'answer'."""
         if self.producers is None:
             raise RuntimeError('FastCaSE was built without producers=...')
         max_len = self.max_dec_len if max_len is None else max_len
@@ -235,50 +291,62 @@ class FastCaSE(_FastModel):
             if mode != 'beam':
                 raise ValueError('n_best needs mode="beam"')
             n_best = _nbest_count(n_best, width)
+        if attribution:
+            self._check_attribution_opt()
         p = self.producers(data['query'], data['passage'])
         d = dict(mem_q=p['mem_q'], mem_p=p['mem_p'], query=data['query'].to(self.weights.device),
                  passage=data['passage'].to(self.weights.device), prior_q=p['prior_q'], prior_p=p['prior_p'],
                  answer_rep=p['answer_rep'], source_map=data['source_map'].to(self.weights.device))
         m = {'beam': L.MODE_BEAM, 'greedy': L.MODE_PROTO_GREEDY, 'module_greedy': L.MODE_MODULE_GREEDY}[mode]
-        if n_best is None:
+        if n_best is None and not attribution:
             return {'answer': self.fast_search(d, max_len, width, m), 'rank': p['rank']}
-        nb = self.fast_search(d, max_len, width, m, nbest=n_best)
-        return {'answer': self.last_engine._finish_tokens(max_len, m), 'rank': p['rank'], 'nbest': nb}
+        got = self.fast_search(d, max_len, width, m, nbest=n_best, attribution=attribution)
+        out = {'answer': self.last_engine._finish_tokens(max_len, m), 'rank': p['rank']}
+        if n_best is not None:
+            out['nbest'] = got.answer if attribution else got
+        if attribution:
+            out['attribution'] = got
+        return out
 
-    def engine_for(self, B, W, S0, S1, T, nbest=1):
-        key = (B, W, S0, S1, T, self.opt, self.n_oov, nbest)
+    def engine_for(self, B, W, S0, S1, T, nbest=1, attribution=False):
+        key = (B, W, S0, S1, T, self.opt, self.n_oov, nbest, bool(attribution))
         if key not in self._engines:
             if len(self._engines) >= 4:
                 self._engines.clear()
             self._engines[key] = CaseDecodeEngine(self.weights, B, W, S0, S1, T, vocab_impl=self.vocab_impl,
-                                                  opt=self.opt, n_oov=self.n_oov, nbest=nbest)
+                                                  opt=self.opt, n_oov=self.n_oov, nbest=nbest, attribution=attribution)
         return self._engines[key]
 
     def encode(self, data):
         return data
 
-    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None):
-        """-> the answers (LongTensor), or with nbest the NBest list of a beam search."""
+    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None,
+                    attribution=False):
+        """-> the answers (LongTensor), with nbest the NBest list of a beam search, with attribution an Attributed."""
+        if attribution:
+            self._check_attribution_opt()
         d = encode_outputs if encode_outputs is not None else data
         B = d['source_map'].size(0)
         S0 = d['mem_q'].reshape(B, -1, L.H).size(1)
         S1 = d['mem_p'].reshape(B, -1, L.H).size(1)
-        eng = self.engine_for(B, width, S0, S1, max_len, nbest or 1)
+        eng = self.engine_for(B, width, S0, S1, max_len, nbest or 1, attribution)
         eng.prefill(d['mem_q'], d['mem_p'], d['query'].ne(0), d['passage'].ne(0), d['prior_q'], d['prior_p'],
                     d['answer_rep'], d['source_map'])
         self.last_engine = eng
-        if nbest is None:
+        if nbest is None and not attribution:
             return eng.decode(max_len, mode, use_graph=self.use_graph)
+        if mode != L.MODE_BEAM and eng.W != 1:
+            raise ValueError('greedy modes need an engine built with W == 1')
         eng.launch(max_len, mode, use_graph=self.use_graph)
-        return eng._finish_nbest()
+        return self._finish(eng, max_len, mode, nbest, attribution)
 
     _KEYS = ('mem_q', 'mem_p', 'query', 'passage', 'prior_q', 'prior_p', 'answer_rep', 'source_map')
 
-    def _prefill_staged(self, d, width, max_len, nbest=1):
+    def _prefill_staged(self, d, width, max_len, nbest=1, attribution=False):
         B = d['source_map'].size(0)
         S0 = d['mem_q'].reshape(B, -1, L.H).size(1)
         S1 = d['mem_p'].reshape(B, -1, L.H).size(1)
-        eng = self.engine_for(B, width, S0, S1, max_len, nbest)
+        eng = self.engine_for(B, width, S0, S1, max_len, nbest, attribution)
         eng.prefill(d['mem_q'], d['mem_p'], d['query'].ne(0), d['passage'].ne(0), d['prior_q'], d['prior_p'],
                     d['answer_rep'], d['source_map'])
         return eng
@@ -300,35 +368,38 @@ class FastGTTP(_FastModel):
         self.opt = int(opt)
         self._engines = {}
 
-    def engine_for(self, B, W, Lc, Lb, T, nbest=1):
-        key = (B, W, Lc, Lb, T, nbest)
+    def engine_for(self, B, W, Lc, Lb, T, nbest=1, attribution=False):
+        key = (B, W, Lc, Lb, T, nbest, bool(attribution))
         if key not in self._engines:
             if len(self._engines) >= 4:
                 self._engines.clear()
             self._engines[key] = GttpDecodeEngine(self.weights, B, W, Lc, Lb, T, vocab_impl=self.vocab_impl,
-                                                  opt=self.opt, nbest=nbest)
+                                                  opt=self.opt, nbest=nbest, attribution=attribution)
         return self._engines[key]
 
-    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None):
-        """-> the answers (LongTensor), or with nbest the NBest list of a beam search."""
+    def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None,
+                    attribution=False):
+        """-> the answers (LongTensor), with nbest the NBest list of a beam search, with attribution an Attributed."""
+        if attribution:
+            self._check_attribution_opt()
         d = dict(data)
         if encode_outputs is not None:
             d.update(encode_outputs)
         if init_decoder_states is not None:
             d['init_state'] = init_decoder_states
-        eng = self._prefill_staged(d, width, max_len, nbest or 1)
+        eng = self._prefill_staged(d, width, max_len, nbest or 1, attribution)
         self.last_engine = eng
-        if nbest is None:
+        if nbest is None and not attribution:
             return eng.decode(max_len, mode, use_graph=self.use_graph)
         eng.launch(max_len, mode, use_graph=self.use_graph)
-        return eng._finish_nbest()
+        return self._finish(eng, max_len, mode, nbest, attribution)
 
     _KEYS = ('context', 'background', 'background_map', 'src_output', 'bg_output', 'init_state')
 
-    def _prefill_staged(self, d, width, max_len, nbest=1):
+    def _prefill_staged(self, d, width, max_len, nbest=1, attribution=False):
         B, Lc = d['context'].shape
         Lb = d['background'].size(1)
-        eng = self.engine_for(B, width, Lc, Lb, max_len, nbest)
+        eng = self.engine_for(B, width, Lc, Lb, max_len, nbest, attribution)
         eng.prefill(d['src_output'], d['bg_output'], d['context'], d['background'], d['background_map'],
                     d['init_state'])
         return eng

@@ -42,6 +42,28 @@ def to_sentence(batch_indices, id2vocab: Dict[int, str]) -> List[List[str]]:
     return out
 
 
+def source_location(source, S0: int, Lp: int):
+    """Attribution source position (``Attributed.source``: an index of CaSE's ``source_map``, the query's S0 positions
+    followed by the passages flattened [NP][Lp], CaSEDataset.py:98-104) -> (memory, passage, offset): (0, -1, s) for a
+    query position, (1, p, o) for offset o of passage p, (-1, -1, -1) for source -1 (pure generation).  Works on an int
+    or elementwise on an integer tensor (then three int64 tensors of its shape)."""
+    if isinstance(source, torch.Tensor):
+        s = source.to(torch.int64)
+        none, query = s < 0, s < S0
+        q = s - S0
+        neg = torch.full_like(s, -1)
+        memory = torch.where(none, neg, torch.where(query, torch.zeros_like(s), torch.ones_like(s)))
+        passage = torch.where(none | query, neg, torch.div(q, Lp, rounding_mode='floor'))
+        offset = torch.where(none, neg, torch.where(query, s, q % Lp))
+        return memory, passage, offset
+    s = int(source)
+    if s < 0:
+        return -1, -1, -1
+    if s < S0:
+        return 0, -1, s
+    return 1, (s - S0) // Lp, (s - S0) % Lp
+
+
 def _cut_point(sent: Sequence, n: int) -> int:
     """The cut ``remove_duplicate_once`` takes for one sentence, or -1: the LARGEST index in [1, len - n] such
     that every element of sent[index:] also occurs in sent[:index]  (common/Utils.py:176-186).

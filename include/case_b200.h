@@ -44,6 +44,17 @@ extern "C" {
 
 typedef void* case_stream_t; /* cudaStream_t */
 
+/* Attribution record of one answer token y chosen from the mixture of its parent prefix (CaSE/Model.py:38-48,
+ * GTTP/Model.py:25-43): part[0] = g0 * softmax(logits)[y] (generation; 0 for dynamic ids >= V and GTTP's masked id 0),
+ * part[1] / part[2] = copy mass of y from memory 0 / memory 1 (CaSE: query / passages; GTTP: part[1] = the background,
+ * part[2] = 0).  The parts sum to the mixture probability p(y).  source = the source position s (index of the
+ * concatenated copy map [memory 0 ; memory 1]) with the largest single contribution gate_i * p_i[s] among positions with
+ * map[s] == y, exact ties to the lowest s; -1 when no position contributes.  The zero record has source -1. */
+typedef struct {
+  float part[3];
+  int32_t source;
+} case_attr_t;
+
 /* select modes (case_beam_select) */
 #define CASE_MODE_MODULE_GREEDY 0 /* CaSE/Model.py:119-122: argmax, no EOS handling          */
 #define CASE_MODE_PROTO_GREEDY 1  /* Generations.py:96-107: EOS->UNK at t0, PAD after the end */
@@ -392,6 +403,10 @@ typedef struct {
    * lie in [V, Vext) - per-query dynamic entries that have no logit, so their mixture value is the copy mass alone -
    * and the top-k indices range over [0, Vext).  0 = V (no extension). */
   int32_t Vext;
+  /* case_sparse_tail only, may be NULL: attribution record (case_attr_t) of every top-k entry, [R][K] like top_vals.  The
+   * copy parts are accumulated in the fixed point of the hash table, so in hash-table mode part[1] + part[2] is exactly the
+   * copy mass the ranking used; with a copy plan they match it to rounding. */
+  case_attr_t* attr;
 } case_tail_args_t;
 int case_row_tail(const case_tail_args_t* a, case_stream_t stream);
 int case_row_tail_max_vocab(void);
@@ -438,6 +453,14 @@ typedef struct {
    * best_len [B][nbest] and out_tokens [B][nbest][Tmax] (PAD initially) hold the entries in rank order; entry 0 is the
    * answer of nbest = 1.  0 or 1: the single best, layouts as above. */
   int32_t nbest;
+  /* attribution (all three or none; NULL = off): attr_cand [R][W] the records of the top-k entries (index as top_vals,
+   * written by case_sparse_tail), attr_hist [R][Tmax+1] the record of the token at (physical row, position) next to tok,
+   * out_attr the records of out_tokens, same layout ([B][Tmax], or [B][nbest][Tmax] for nbest > 1; zero records with
+   * source -1 initially).  Greedy: an EOS rewritten to UNK at t = 0 keeps its record, PAD after the end gets the zero
+   * record. */
+  const case_attr_t* attr_cand;
+  case_attr_t* attr_hist;
+  case_attr_t* out_attr;
 } case_select_args_t;
 
 int case_beam_select(const case_select_args_t* a, case_stream_t stream);
@@ -578,6 +601,11 @@ typedef struct {
   int32_t n_oov;
   int32_t* tok_ext;
   int32_t nbest;                        /* n-best list of the beam search (case_select_args_t.nbest); 0 or 1: the best only */
+  /* attribution records of the search (case_select_args_t.attr_*; all three or none, NULL = off): attr_cand [R][W],
+   * attr_hist [R][Tmax+1], out_attr like out_tokens.  Only the sparse tail computes them: a request on a step that would
+   * not take it (CASE_OPT_DENSE_TAIL / CASE_OPT_UNFUSED_TAIL, materialize_only, no base_* buffers, V < 2W, more than
+   * case_sparse_tail_max_sources() source positions) is refused before the first launch. */
+  case_attr_t* attr_cand; case_attr_t* attr_hist; case_attr_t* out_attr;
 } case_step_args_t;
 
 /* Enqueue one full decode step t (embedding .. select) for all R rows: the body of the eval loop
@@ -612,6 +640,9 @@ typedef struct {
    * handle's side stream beside the attention over the background (CASE_OPT_NO_FORK switches it off) */
   case_fork_t* fork; float* qa1;
   int32_t nbest;                                         /* n-best list of the beam search (case_select_args_t.nbest) */
+  /* attribution records (as in case_step_args_t; part[1] = copy from the background, part[2] = 0); refused before the
+   * first launch unless the step takes the sparse tail */
+  case_attr_t* attr_cand; case_attr_t* attr_hist; case_attr_t* out_attr;
 } gttp_step_args_t;
 
 /* One GTTP decode step (GTTP/Model.py:176-193 -> BBCDecoder.forward :113-131 ->
