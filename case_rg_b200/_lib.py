@@ -76,6 +76,22 @@ class TailArgs(C.Structure):
                 ('cp_n', vp), ('cp_uid', vp), ('cp_first', vp), ('cp_start', vp), ('cp_perm', vp), ('Vext', i32),
                 ('attr', vp)]
 
+    def __init__(self, *args, **kw):
+        # the launchers read every block as the complete case_tail_args_t: a block built as TailArgs gets the storage of
+        # the trailing constraint fields too (zero: no constraints)
+        super().__init__(*args, **kw)
+        size, full = C.sizeof(type(self)), C.sizeof(TailConstrArgs)
+        if size < full:
+            C.resize(self, full)
+            C.memset(C.addressof(self) + size, 0, full - size)
+
+
+# The search constraints trail the argument blocks (ABI version 2 unchanged), appended by subclassing like the attribution
+# pointers: TailConstrArgs / StepConstrArgs / GttpStepConstrArgs are the complete blocks the launchers read.
+class TailConstrArgs(TailArgs):
+    _fields_ = [('hist_tok', vp), ('hist_anc', vp)] + \
+               [(n, i32) for n in ('hist_ld', 't', 'eos', 'no_repeat_ngram', 'min_len')]
+
 
 class StepArgs(C.Structure):
     _fields_ = [(n, i32) for n in ('B', 'W', 'R', 'V', 'ldv', 'Tmax', 'dtype', 'fast_tanh', 'vocab_impl', 'mode')] + \
@@ -97,6 +113,10 @@ class StepAttrArgs(StepArgs):
     _fields_ = [('attr_cand', vp), ('attr_hist', vp), ('out_attr', vp)]
 
 
+class StepConstrArgs(StepAttrArgs):
+    _fields_ = [('no_repeat_ngram', i32), ('min_len', i32)]
+
+
 class GttpStepArgs(C.Structure):
     _fields_ = [(n, i32) for n in ('B', 'W', 'R', 'V', 'ldv', 'dtype', 'fast_tanh', 'vocab_impl', 'mode', 'Lc', 'Lb',
                                    'nsplit_c', 'nsplit_b', 'max_len', 'BOS', 'EOS', 'UNK', 'PAD',
@@ -114,6 +134,10 @@ class GttpStepArgs(C.Structure):
 
 class GttpStepAttrArgs(GttpStepArgs):
     _fields_ = [('attr_cand', vp), ('attr_hist', vp), ('out_attr', vp)]
+
+
+class GttpStepConstrArgs(GttpStepAttrArgs):
+    _fields_ = [('no_repeat_ngram', i32), ('min_len', i32)]
 
 
 # name -> argtypes (return type is int for all but the three listed below)
@@ -175,7 +199,7 @@ _PROTOS = {
 _SIZE_FNS = ['case_vocab_tc_workspace_bytes', 'case_vocab_tc_packed_weight_bytes']
 _SIZE_FNS2 = ['case_interaction_smem_bytes', 'case_gemm_rows_packed_weight_bytes']      # (int, int) -> size_t
 EXPORTS = sorted(list(_PROTOS) + ['case_abi_version', 'case_last_error', 'case_struct_size'] + _SIZE_FNS + _SIZE_FNS2)
-_STRUCTS = [Seg, RowLinArgs, LayerWeights, SelectAttrArgs, StepAttrArgs, GttpStepAttrArgs, TailArgs, ChainPost]
+_STRUCTS = [Seg, RowLinArgs, LayerWeights, SelectAttrArgs, StepConstrArgs, GttpStepConstrArgs, TailConstrArgs, ChainPost]
 
 _lib = None
 

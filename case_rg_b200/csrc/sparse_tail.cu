@@ -138,14 +138,53 @@ __global__ __launch_bounds__(ST) void vocab_base_kernel(const float* __restrict_
 __device__ __forceinline__ uint32_t sp_hash(int id, int shift) { return ((uint32_t)id * 2654435761u) >> shift; }
 __device__ __forceinline__ uint32_t sp_step(int id) { return (((uint32_t)id * 40503u) >> 4) | 1u; }
 
+// slot of id in the row's touched-id table, -1 if untouched: binary search of the sorted list (plan mode) or the probe
+// sequence of the hash table
+__device__ __forceinline__ int sp_find(const int* hkeys, int nent, bool plan, int id, int hshift, uint32_t hmask) {
+  if (plan) {
+    int lo = 0, hi = nent;
+    while (lo < hi) {
+      const int mid = (lo + hi) >> 1;
+      if (hkeys[mid] < id) lo = mid + 1; else hi = mid;
+    }
+    return lo < nent && hkeys[lo] == id ? lo : -1;
+  }
+  uint32_t slot = sp_hash(id, hshift);
+  const uint32_t step = sp_step(id);
+  while (true) {
+    const int key = hkeys[slot];
+    if (key == id) return (int)slot;
+    if (key == -1) return -1;
+    slot = (slot + step) & hmask;
+  }
+}
+
+// Constrained launches (case_tail_args_t.no_repeat_ngram / min_len) append these int arrays to the dynamic shared memory,
+// after the table: the row's answer so far, the ban candidates, the banned ids (one entry per candidate, -1 = none or a
+// repeat of an earlier candidate) and the row's base entries
+constexpr int CS_HIST = 0, CS_CAND = CS_HIST + CASE_MAX_T, CS_BAN = CS_CAND + CASE_MAX_T + 1,
+              CS_BASE = CS_BAN + CASE_MAX_T + 1, CS_INTS = CS_BASE + 2 * SP_PARTS * 2 * CASE_MAX_W;
+
+__device__ __forceinline__ bool sp_banned(const int* ban, int nban, int id) {
+  bool hit = false;
+  for (int i = 0; i < nban; ++i) hit |= ban[i] == id;
+  return hit;
+}
+
 // ATTR (case_tail_args_t.attr != NULL): after the top-k, an attribution pass writes the record of every winner (see
-// below); the fused select then carries the records with the tokens
-template <bool ATTR>
+// below); the fused select then carries the records with the tokens.
+// CONSTR (no_repeat_ngram or min_len set): the row's banned ids leave the candidate set.  A banned touched id is looked
+// up once and its value set to -inf; a banned base entry is not offered.  Exactness: an untouched id enters the top-K
+// through the base entries only, and the unconstrained argument needs 2K of them (K for the result, K of slack for the
+// ties of the gate scale's rounding).  A banned base entry uses up one of them, so with a = the allowed ids among the
+// row's global top-k2 base entries the row keeps the usual path while a >= 2K and otherwise takes an exact pass over
+// all V logits (offering every allowed untouched id; fbcount counts these rows).
+template <bool ATTR, bool CONSTR>
 __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t a, const float* __restrict__ base_ms,
                                                          const float* __restrict__ base_e,
                                                          const int32_t* __restrict__ base_i, int k2, int nslots,
                                                          long long* dbg, const case_select_args_t sel, int do_select,
-                                                         int32_t* __restrict__ qcount) {
+                                                         int32_t* __restrict__ qcount, int* fbcount) {
   // [nslots] ids (-1 = empty), then [nslots] low words of the masses (later: the final float values), then - hash
   // mode only - [nslots] high words.  The copy mass of an id is accumulated as a 64-bit FIXED-POINT integer (2^-48
   // units, two native 32-bit shared-memory atomics with an explicit carry): integer addition is associative, so the
@@ -182,6 +221,16 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
   }
   pdl_wait();
   stamp();
+  // constrained: the row's answer y_1 .. y_t, gathered along its ancestry like the select writes a finished path (the
+  // previous step's select wrote it)
+  int* const cs = hkeys + (plan ? 2 : 3) * nslots;
+  if constexpr (CONSTR) {
+    for (int j = tid; j < a.t; j += TS) {
+      const int p = j + 1;
+      const int src = p == a.t ? r : a.hist_anc[(size_t)r * a.hist_ld + p];
+      cs[CS_HIST + j] = a.hist_tok[(size_t)src * a.hist_ld + p];
+    }
+  }
   float g0, F[2] = {0.f, 0.f}, M[2] = {0.f, 0.f};
   if (a.do_finalize) {
     // every thread merges the split statistics itself (a few broadcast loads), column tid of the contexts
@@ -304,6 +353,33 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
       }
     }
     __syncthreads();       // the table is initialised
+  }
+  if constexpr (CONSTR) {
+    // (both branches above end with a barrier: the history is visible.)  Candidate j < t: the n-gram y_{j+1} ..
+    // y_{j+n} lies in the answer and its first n - 1 tokens are the answer's last n - 1, so y_{j+n} is banned;
+    // candidate t: the EOS of an answer shorter than min_len.  An id is kept at its first candidate only
+    const int t = a.t, n = a.no_repeat_ngram;
+    if (tid <= t) {
+      int c = -1;
+      if (tid < t) {
+        if (n > 0 && tid + n <= t) {
+          bool eq = true;
+          for (int k = 0; k < n - 1; ++k) eq &= cs[CS_HIST + tid + k] == cs[CS_HIST + t - n + 1 + k];
+          if (eq) c = cs[CS_HIST + tid + n - 1];
+        }
+      } else if (t < a.min_len) {
+        c = a.eos;
+      }
+      cs[CS_CAND + tid] = c;
+    }
+    __syncthreads();
+    if (tid <= t) {
+      const int c = cs[CS_CAND + tid];
+      bool first = c >= 0;
+      for (int j = 0; j < tid; ++j) first &= cs[CS_CAND + j] != c;
+      cs[CS_BAN + tid] = first ? c : -1;
+    }
+    // (visible after the barrier that ends the copy-mass pass)
   }
   stamp();
   // ---- copy mass of both memories into the hash table (double hashing, ids are exact).  The source positions of
@@ -451,6 +527,20 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
     }
   }
   stamp();
+  const int nban = a.t + 1;                              // constrained: entries of the banned list
+  if constexpr (CONSTR) {
+    // banned touched ids: one lookup each, the value becomes -inf; then the thread maxima again without them
+    __syncthreads();
+    if (tid < nban) {
+      const int id = cs[CS_BAN + tid];
+      const int sl = id >= 0 ? sp_find(hkeys, nent, plan, id, hshift, hmask) : -1;
+      if (sl >= 0) hvals[sl] = -INFINITY;
+    }
+    __syncthreads();
+    tmax = -INFINITY;
+    for (int sl = tid; sl < nent; sl += TS)
+      if (hkeys[sl] >= 0) tmax = fmaxf(tmax, hvals[sl]);
+  }
   float fb = -INFINITY;                                  // base candidates that received no copy mass
   int idb = 0x7fffffff;
   if (tid < SP_PARTS * k2) {
@@ -475,9 +565,58 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
           slot = (slot + step) & hmask;
         }
       }
-      if (!found) { fb = scl * sp_exp(l - mm); idb = id; }
+      if (!found && !(CONSTR && sp_banned(cs + CS_BAN, nban, id))) { fb = scl * sp_exp(l - mm); idb = id; }
     }
   }
+  bool exact = false;
+  if constexpr (CONSTR) {
+    // a = allowed ids among the row's global top-k2 base entries (rank over the SP_PARTS * k2 partial entries)
+    int* bi = cs + CS_BASE;
+    float* bl = reinterpret_cast<float*>(bi + SP_PARTS * k2);
+    int id = 0x7fffffff;
+    float l = -INFINITY;
+    if (tid < SP_PARTS * k2) {
+      id = base_i[(size_t)r * SP_PARTS * k2 + tid];
+      l = base_e[(size_t)r * SP_PARTS * k2 + tid];
+      if (!((unsigned)id < (unsigned)V && l > -INFINITY)) { id = 0x7fffffff; l = -INFINITY; }
+      bi[tid] = id;
+      bl[tid] = l;
+    }
+    __syncthreads();
+    bool allowed = false;
+    if (tid < SP_PARTS * k2 && l > -INFINITY) {
+      int rank = 0;
+      for (int j = 0; j < SP_PARTS * k2; ++j) rank += tk_better(bl[j], bi[j], l, id);
+      allowed = rank < k2 && !sp_banned(cs + CS_BAN, nban, id);
+    }
+    exact = __syncthreads_count(allowed) < 2 * K;
+  }
+  float ov = -INFINITY;
+  int oi = 0x7fffffff;
+  if (CONSTR && exact) {
+    // exact pass: every allowed touched id (banned ones hold -inf) and every allowed untouched id of the row
+    if (fbcount != nullptr && tid == 0) atomicAdd(fbcount, 1);
+    WarpTopK wl;
+    wl.init();
+    for (int s0 = 0; s0 < nent; s0 += TS) {
+      const int id = s0 + tid < nent ? hkeys[s0 + tid] : -1;
+      const float v = id >= 0 ? hvals[s0 + tid] : -INFINITY;
+      wl.offer(K, v, v > -INFINITY ? id : 0x7fffffff);
+    }
+    for (int v0 = 0; v0 < V; v0 += TS) {
+      const int id = v0 + tid;
+      float f = -INFINITY;
+      if (id < V && !(a.mask_col0 && id == 0) && sp_find(hkeys, nent, plan, id, hshift, hmask) < 0 &&
+          !sp_banned(cs + CS_BAN, nban, id)) {
+        const float l = x[id];
+        if (l > -INFINITY) f = scl * sp_exp(l - mm);
+      }
+      wl.offer(K, f, f > -INFINITY ? id : 0x7fffffff);
+    }
+    block_merge_lists(sc, wl, K);
+    ov = wl.ev; oi = wl.ei;
+    stamp();
+  } else {
   tmax = fmaxf(tmax, fb);
   const float T = block_kth_max(sc, K, tmax);
   if (tmax >= T && tmax > -INFINITY) {
@@ -489,8 +628,6 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
   }
   __syncthreads();
   stamp();
-  float ov = -INFINITY;
-  int oi = 0x7fffffff;
   if (!block_select(sc, K, ov, oi)) {                    // massive ties: offer every candidate
     WarpTopK wl;
     wl.init();
@@ -501,6 +638,7 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
     wl.offer(K, fb, idb);
     block_merge_lists(sc, wl, K);
     ov = wl.ev; oi = wl.ei;
+  }
   }
   if (warp == 0 && lane < K) {
     a.top_vals[(size_t)r * K + lane] = ov;
@@ -616,6 +754,10 @@ extern "C" int case_vocab_base(const float* logits, int ldl, int R, int V, int m
 
 static thread_local long long* g_sp_dbg = nullptr;   // debugging aid of the calling thread
 extern "C" int case_debug_sparse_tail_timing(void* buf) { g_sp_dbg = (long long*)buf; return 0; }
+// debugging aid: every constrained row that takes the exact pass over its logits adds 1 to *counter (int32 on the
+// device; NULL = off).  Read at launch, so a CUDA graph keeps the pointer it was captured with
+static thread_local int* g_sp_fallbacks = nullptr;
+extern "C" int case_debug_sparse_tail_fallbacks(void* counter) { g_sp_fallbacks = (int*)counter; return 0; }
 
 extern "C" int case_sparse_tail_max_sources(void) { return 10900; }   // 16384 slots at load factor <= 2/3
 
@@ -641,7 +783,7 @@ extern "C" int case_sparse_tail(const case_tail_args_t* a, const float* base_ms,
   CB_REQUIRE(!plan || (a->nmem == 2 && a->cp_uid && a->cp_first && a->cp_start && a->cp_perm && a->cp_ld >= total && total < 65536),
              "case_sparse_tail: the copy plan needs cp_uid / cp_first / cp_start / cp_perm with cp_ld >= S0 + S1 (two memories, < 65536 positions)");
   // plan mode: (id, value) per list entry, at most one per source position; the hash layout otherwise
-  const size_t smem = plan ? (size_t)((total + 3) / 4 * 4) * 8 : (size_t)nslots * 12;
+  size_t smem = plan ? (size_t)((total + 3) / 4 * 4) * 8 : (size_t)nslots * 12;
   if (plan) nslots = (total + 3) / 4 * 4;
   if (sel) {
     int rc = check_nbest(sel->nbest, sel->W, sel->mode);
@@ -651,16 +793,33 @@ extern "C" int case_sparse_tail(const case_tail_args_t* a, const float* base_ms,
     CB_REQUIRE((sel->out_attr != nullptr) == (a->attr != nullptr) && (sel->attr_cand == nullptr || sel->attr_cand == a->attr),
                "case_sparse_tail: a fused select with attribution needs attr_cand == the tail's attr (both on or both off)");
   }
+  const bool constr = a->no_repeat_ngram != 0 || a->min_len != 0;
+  if (constr) {
+    CB_REQUIRE(a->no_repeat_ngram >= 0 && a->no_repeat_ngram <= CASE_MAX_T && a->min_len >= 0 && a->min_len < CASE_MAX_T,
+               "case_sparse_tail: no_repeat_ngram must be 0..CASE_MAX_T and min_len 0..CASE_MAX_T-1");
+    CB_REQUIRE(a->hist_tok && a->hist_anc && a->t >= 0 && a->t < CASE_MAX_T && a->hist_ld > a->t,
+               "case_sparse_tail: constraints need the answer history (hist_tok, hist_anc, 0 <= t < hist_ld)");
+    CB_REQUIRE(a->V >= 2 * a->K + a->hist_ld, "case_sparse_tail: constraints need V >= 2K + Tmax + 1 (hist_ld = Tmax + 1)");
+    smem += (size_t)CS_INTS * 4;
+  }
   const bool attr = a->attr != nullptr;
   cudaStream_t st = (cudaStream_t)stream;
-  if (attr) ensure_smem<sparse_tail_kernel<true>>(16384 * 12);
-  else ensure_smem<sparse_tail_kernel<false>>(16384 * 12);
+  constexpr int cx = CS_INTS * 4;
+  if (constr) {
+    if (attr) ensure_smem<sparse_tail_kernel<true, true>>(16384 * 12 + cx);
+    else ensure_smem<sparse_tail_kernel<false, true>>(16384 * 12 + cx);
+  } else {
+    if (attr) ensure_smem<sparse_tail_kernel<true, false>>(16384 * 12);
+    else ensure_smem<sparse_tail_kernel<false, false>>(16384 * 12);
+  }
   CB_REQUIRE(sel == nullptr || (qcount != nullptr && sel->B * sel->W == a->R && sel->W == a->W && a->K == a->W),
              "case_sparse_tail: fused select needs qcount and matching B / W (k = W)");
   case_select_args_t sv;
   memset(&sv, 0, sizeof(sv));
   if (sel) sv = *sel;
-  launch_k(attr ? sparse_tail_kernel<true> : sparse_tail_kernel<false>, a->R, TS, smem, st, *a, base_ms, base_e, base_i, k2,
-           nslots, g_sp_dbg, sv, sel ? 1 : 0, qcount);
+  auto kern = constr ? (attr ? sparse_tail_kernel<true, true> : sparse_tail_kernel<false, true>)
+                     : (attr ? sparse_tail_kernel<true, false> : sparse_tail_kernel<false, false>);
+  launch_k(kern, a->R, TS, smem, st, *a, base_ms, base_e, base_i, k2, nslots, g_sp_dbg, sv, sel ? 1 : 0, qcount,
+           g_sp_fallbacks);
   return check_launch("case_sparse_tail");
 }

@@ -145,6 +145,37 @@ static int check_step_attr(const case_attr_t* cand, const case_attr_t* hist, con
   return 0;
 }
 
+// Search constraints of a step (no_repeat_ngram / min_len of the step blocks; both 0 = off): in range, in a search mode
+// that has them, and only where the step takes the sparse tail - the only tail that applies them.  Checked before the
+// first launch of the step, after the n-best and attribution checks.
+static int check_step_constr(int n, int min_len, int mode, int max_len, int V, int W, int Tmax, bool sparse,
+                             const char* what) {
+  if (n == 0 && min_len == 0) return 0;
+  char msg[256];
+  const char* why = nullptr;
+  if (n < 0 || n > max_len || min_len < 0 || min_len >= max_len)
+    why = "constraints out of range: 0 <= no_repeat_ngram <= max_len, 0 <= min_len < max_len";
+  else if (mode != CASE_MODE_BEAM && mode != CASE_MODE_PROTO_GREEDY)
+    why = "constraints need CASE_MODE_BEAM or CASE_MODE_PROTO_GREEDY";
+  else if (!sparse)
+    why = "constraints need the sparse tail (not with CASE_OPT_DENSE_TAIL / UNFUSED_TAIL, materialize_only, missing "
+          "base_* buffers, V < 2W or too many source positions)";
+  else if (V < 2 * W + Tmax + 1)
+    why = "constraints need V >= 2W + Tmax + 1";
+  if (why == nullptr) return 0;
+  snprintf(msg, sizeof(msg), "%s: %s", what, why);
+  set_error(msg);
+  return CASE_EINVAL;
+}
+
+// the tail's view of the search state: row r's answer tokens along anc_in (the returned ids: tok_ext when present)
+static void set_tail_constr(case_tail_args_t& ta, const int32_t* tok, const int32_t* anc_in, int TL, int t, int EOS,
+                            int n, int min_len) {
+  if (n == 0 && min_len == 0) return;
+  ta.hist_tok = tok; ta.hist_anc = anc_in; ta.hist_ld = TL; ta.t = t; ta.eos = EOS;
+  ta.no_repeat_ngram = n; ta.min_len = min_len;
+}
+
 static void set_select_attr(case_select_args_t& s, case_attr_t* cand, case_attr_t* hist, case_attr_t* out) {
   if (out == nullptr) return;
   s.attr_cand = cand; s.attr_hist = hist; s.out_attr = out;
@@ -177,7 +208,10 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
   const bool sparse = use_tail == 2 && !a->materialize_only && a->base_ms && a->base_e && a->base_i && a->V >= k2 &&
                       a->S[0] + a->S[1] <= case_sparse_tail_max_sources();
   TRY(check_step_attr(a->attr_cand, a->attr_hist, a->out_attr, sparse, "case_decode_step"));
+  TRY(check_step_constr(a->no_repeat_ngram, a->min_len, a->mode, a->max_len, a->V, W, a->Tmax, sparse, "case_decode_step"));
   const bool attr = a->out_attr != nullptr;
+  // constrained steps ask vocab_base for the most base entries the buffers hold (see sparse_tail.cu: exactness)
+  const int k2b = (a->no_repeat_ngram || a->min_len) ? 2 * CASE_MAX_W : k2;
   // gate form of the additive attentions: the contexts only feed the mixture gate, so 3 gate-projected numbers
   // per key replace the value rows (needs the sparse tail, which merges gate partials instead of contexts)
   const bool gate = !(opt & CASE_OPT_NO_GATE) && sparse && dt == CASE_BF16 && a->Gv[0] != nullptr && a->Gv[1] != nullptr;
@@ -321,7 +355,7 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
       TRY(gen0());
     }
     TRY(case_vocab_gemm(a->gfeat, a->Wv, nullptr, a->logits, R, a->V, a->ldv, dt, a->vocab_impl, a->vocab_ws, st));
-    if (sparse) TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 0, k2, a->base_ms, a->base_e, a->base_i, st));
+    if (sparse) TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 0, k2b, a->base_ms, a->base_e, a->base_i, st));
     if (fork) {
       CUTRY(cudaStreamWaitEvent(st, ev_join[0], 0));
       CUTRY(cudaStreamWaitEvent(st, ev_join[1], 0));
@@ -349,7 +383,7 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
   TRY(case_layernorm_rows(a->h, a->lnN_g, a->lnN_b, a->hN, R, st));
   TRY(gen0());
   TRY(case_vocab_gemm(a->gfeat, a->Wv, nullptr, a->logits, R, a->V, a->ldv, dt, a->vocab_impl, a->vocab_ws, st));
-  if (sparse) TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 0, k2, a->base_ms, a->base_e, a->base_i, st));
+  if (sparse) TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 0, k2b, a->base_ms, a->base_e, a->base_i, st));
   }
   if (sparse || (use_tail && n_oov == 0 && a->V <= case_row_tail_max_vocab())) {
     // one launch: attention merge + gates, softmax x gate, both copy scatters, top-k; the [R, V]
@@ -380,7 +414,8 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
                                            a->ended, a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
       if (n_oov) { sel.V_in = a->V; sel.tok_ext = a->tok_ext; }
       set_select_attr(sel, a->attr_cand, a->attr_hist, a->out_attr);
-      TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2, fuse_sel ? &sel : nullptr, a->qcount, st));
+      set_tail_constr(ta, n_oov ? a->tok_ext : a->tok, anc, TL, t, a->EOS, a->no_repeat_ngram, a->min_len);
+      TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2b, fuse_sel ? &sel : nullptr, a->qcount, st));
       if (fuse_sel) return 0;
     } else {
       TRY(case_row_tail(&ta, st));
@@ -437,6 +472,8 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
   const bool sparse = use_tail && !(opt & CASE_OPT_DENSE_TAIL) && !a->materialize_only && a->base_ms && a->base_e && a->base_i &&
                       a->V >= k2 && a->Lb <= case_sparse_tail_max_sources();
   TRY(check_step_attr(a->attr_cand, a->attr_hist, a->out_attr, sparse, "gttp_decode_step"));
+  TRY(check_step_constr(a->no_repeat_ngram, a->min_len, a->mode, a->max_len, a->V, W, a->Tmax, sparse, "gttp_decode_step"));
+  const int k2b = (a->no_repeat_ngram || a->min_len) ? 2 * CASE_MAX_W : k2;   // as in case_decode_step
 
   TRY(case_embed_rows(a->E, nullptr, a->tok, TL, t, 1.0f, a->emb, R, st));
   // two additive attentions with the previous GRU state as query (GTTP/Model.py:117-122)
@@ -503,7 +540,7 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
   TRY(case_vocab_gemm(a->feat, a->Wv, a->bv, a->logits, R, a->V, a->ldv, dt, a->vocab_impl, a->vocab_ws, st));
   TRY(case_gttp_gates(a->feat, a->wc, a->bc, a->gates, a->fac, CASE_MAX_SPLIT, ns[1], R, st));
   if (sparse) {
-    TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 1, k2, a->base_ms, a->base_e, a->base_i, st));
+    TRY(case_vocab_base(a->logits, a->ldv, R, a->V, 1, k2b, a->base_ms, a->base_e, a->base_i, st));
     case_tail_args_t ta;
     memset(&ta, 0, sizeof(ta));
     ta.R = R; ta.V = a->V; ta.W = W; ta.K = W; ta.ldl = a->ldv; ta.ldd = a->ldv; ta.mask_col0 = 1; ta.nmem = 1;
@@ -512,7 +549,8 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
     ta.S[0] = a->Lb; ta.attn_un[0] = a->attn_un[1];
     ta.top_vals = a->top_vals; ta.top_idx = a->top_idx;
     ta.attr = a->attr_cand;
-    TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2, nullptr, nullptr, st));
+    set_tail_constr(ta, a->tok, a->anc[t & 1], TL, t, a->EOS, a->no_repeat_ngram, a->min_len);
+    TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2b, nullptr, nullptr, st));
   } else if (use_tail && a->V <= case_row_tail_max_vocab()) {
     case_tail_args_t ta;
     memset(&ta, 0, sizeof(ta));

@@ -362,6 +362,30 @@ def check_attribution(opt: int, V: int, W: int, nsources: int) -> None:
                          f'{L.load().case_sparse_tail_max_sources()}')
 
 
+def check_constraints(opt: int, V: int, W: int, nsources: int, Tmax: int, no_repeat_ngram: int, min_len: int,
+                      max_len: Optional[int] = None, mode: Optional[int] = None) -> None:
+    """Search constraints (no_repeat_ngram / min_len, 0 = off) are applied by the sparse tail only: ValueError for a
+    request the step would refuse.  max_len / mode: also check them against one decode."""
+    n, m = int(no_repeat_ngram), int(min_len)
+    if n == 0 and m == 0:
+        return
+    lim = Tmax if max_len is None else max_len
+    if not 0 <= n <= lim:
+        raise ValueError(f'no_repeat_ngram must be 0..max_len ({lim}), got {n}')
+    if not 0 <= m < lim:
+        raise ValueError(f'min_len must be 0..max_len - 1 ({lim - 1}), got {m}')
+    if mode is not None and mode not in (L.MODE_BEAM, L.MODE_PROTO_GREEDY):
+        raise ValueError('no_repeat_ngram / min_len apply to the beam and greedy searches (not module_greedy)')
+    if opt & (L.OPT_DENSE_TAIL | L.OPT_UNFUSED_TAIL):
+        raise ValueError('no_repeat_ngram / min_len need the sparse tail: not with OPT_DENSE_TAIL / OPT_UNFUSED_TAIL')
+    if V < 2 * W + Tmax + 1:
+        raise ValueError(f'no_repeat_ngram / min_len need V >= 2 * width + max_target_length + 1 (V = {V}, width = {W}, '
+                         f'max_target_length = {Tmax})')
+    if nsources > L.load().case_sparse_tail_max_sources():
+        raise ValueError(f'no_repeat_ngram / min_len need the sparse tail: {nsources} source positions exceed its '
+                         f'{L.load().case_sparse_tail_max_sources()}')
+
+
 class _SearchState:
     """Buffers shared by both engines for the on-device greedy / beam bookkeeping.  nbest > 1: the beam search keeps
     the nbest best finished hypotheses of every query (best_key / best_len [B, nbest], out_tokens [B, nbest, Tmax]).
@@ -441,6 +465,11 @@ class _EngineBase:
     # takes it as a uint8 view of the ctypes struct - and the stream is torch's current stream either way.
     use_torch_ops = False
 
+    def _check_launch_constraints(self, max_len: int, mode: int) -> None:
+        n, m = self.constraints
+        if n or m:
+            check_constraints(int(self.args.opt), self.V, self.W, 0, self.Tmax, n, m, max_len, mode)
+
     def _step(self, t: int, cuda_stream: int):
         if self.use_torch_ops:
             ops = L.load_torch_ops()
@@ -497,16 +526,21 @@ class CaseDecodeEngine(_EngineBase):
 
     def __init__(self, weights: CaseWeights, B: int, W: int, S0: int, S1: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0, n_oov: int = 0, nbest: int = 1, attribution: bool = False):
+                 opt: int = 0, n_oov: int = 0, nbest: int = 1, attribution: bool = False, no_repeat_ngram: int = 0,
+                 min_len: int = 0):
         """n_oov > 0: extended vocabulary - ``source_map`` entries in [V, V + n_oov) are per-query dynamic (OOV) words,
         the mixture and its top-k range over V + n_oov ids (pointer-generator extension; an OOV id is fed back as UNK).
         nbest (1..W): a beam decode keeps the nbest best finished hypotheses per query (read with ``_finish_nbest``).
-        attribution: every decode also records where each answer token came from (read with ``_finish_attribution``)."""
+        attribution: every decode also records where each answer token came from (read with ``_finish_attribution``).
+        no_repeat_ngram / min_len: search constraints of every beam / greedy decode (0 = off; see
+        generations.beam): no answer repeats an n-gram, EOS is banned before step min_len."""
         self.opt, self.n_oov = int(opt), int(n_oov)
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
         if attribution:
             check_attribution(self.opt, weights.V, W, S0 + S1)
+        check_constraints(self.opt, weights.V, W, S0 + S1, Tmax, no_repeat_ngram, min_len)
+        self.constraints = (int(no_repeat_ngram), int(min_len))
         self.nparts = 3
         if not (1 <= Tmax <= L.MAX_T):
             raise ValueError(f'max_target_length must be 1..{L.MAX_T}')
@@ -605,7 +639,8 @@ class CaseDecodeEngine(_EngineBase):
         self._fill_args()
 
     def _fill_args(self):
-        a = self.args = L.StepAttrArgs()
+        a = self.args = L.StepConstrArgs()
+        a.no_repeat_ngram, a.min_len = self.constraints
         w = self.w
         a.opt, a.fork = self.opt, self._fork.h
         if self.n_oov:
@@ -742,6 +777,7 @@ class CaseDecodeEngine(_EngineBase):
         read later with ``_finish_tokens``); lets several engines decode concurrently on several streams."""
         if max_len > self.Tmax:
             raise ValueError('max_len exceeds the engine Tmax')
+        self._check_launch_constraints(max_len, mode)
         self.args.mode, self.args.max_len, self.args.materialize_only = mode, max_len, 0
         self.ensure_graph(max_len, mode, use_graph)
         self.state.reset()
@@ -760,6 +796,8 @@ class CaseDecodeEngine(_EngineBase):
     def step_distribution(self, t: int) -> torch.Tensor:
         """Protocol ``generate`` face: run step t up to the finished distribution and return a view
         [R, V] of it (no top-k / select); the caller drives tok/anc through ``state``."""
+        if any(self.constraints):
+            raise ValueError('no_repeat_ngram / min_len apply to the beam and greedy searches, not to the `generate` face')
         for i in range(2):
             if self._mv_src[i] is not None:
                 self.Mv[i].copy_(self._mv_src[i].view_as(self.Mv[i]))
@@ -819,11 +857,13 @@ class GttpWeights:
 class GttpDecodeEngine(_EngineBase):
     def __init__(self, weights: GttpWeights, B: int, W: int, Lc: int, Lb: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0, nbest: int = 1, attribution: bool = False):
+                 opt: int = 0, nbest: int = 1, attribution: bool = False, no_repeat_ngram: int = 0, min_len: int = 0):
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
         if attribution:
             check_attribution(int(opt), weights.V, W, Lb)
+        check_constraints(int(opt), weights.V, W, Lb, Tmax, no_repeat_ngram, min_len)
+        self.constraints = (int(no_repeat_ngram), int(min_len))
         self.nparts = 2
         self.w = weights
         self.device = dev = weights.device
@@ -863,7 +903,8 @@ class GttpDecodeEngine(_EngineBase):
         self._graphs = {}
         self._step_fn = L.load().gttp_decode_step
         self._step_name = 'gttp_decode_step'
-        a = self.args = L.GttpStepAttrArgs()
+        a = self.args = L.GttpStepConstrArgs()
+        a.no_repeat_ngram, a.min_len = self.constraints
         w = weights
         a.B, a.W, a.R, a.V, a.ldv, a.dtype = B, W, R, V, self.ldv, w.cdtype
         a.opt = int(opt)
@@ -918,6 +959,7 @@ class GttpDecodeEngine(_EngineBase):
             raise ValueError('max_len exceeds the engine Tmax')
         if mode != L.MODE_BEAM and self.W != 1:
             raise ValueError('greedy modes need an engine built with W == 1')
+        self._check_launch_constraints(max_len, mode)
         self.args.mode, self.args.max_len, self.args.materialize_only = mode, max_len, 0
         self._reset()
         if use_graph and (max_len, mode) not in self._graphs:

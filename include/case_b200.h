@@ -407,6 +407,17 @@ typedef struct {
    * copy parts are accumulated in the fixed point of the hash table, so in hash-table mode part[1] + part[2] is exactly the
    * copy mass the ranking used; with a copy plan they match it to rounding. */
   case_attr_t* attr;
+  /* case_sparse_tail only: search constraints (no_repeat_ngram = min_len = 0: off, the fields below are ignored).
+   * Row r is at step t (0 <= t < CASE_MAX_T) and its answer so far is y_1 .. y_t, position j held by
+   * hist_tok[((j == t) ? r : hist_anc[r][j])][j] (rows of hist_ld >= t + 1 ints; the select's tok / tok_ext and anc_in).
+   * no_repeat_ngram = n (1..CASE_MAX_T): an id y with (y_{t-n+2} .. y_t, y) already a contiguous n-gram of y_1 .. y_t
+   * is banned; min_len = m (0..CASE_MAX_T-1): eos is banned while t < m.  Banned ids leave the candidate set and nothing
+   * is renormalised: top_vals / top_idx are the exact top-K of the mixture restricted to the allowed ids.  Needs
+   * V >= 2K + hist_ld, so K allowed ids always exist. */
+  const int32_t* hist_tok;
+  const int32_t* hist_anc;
+  int32_t hist_ld, t, eos;
+  int32_t no_repeat_ngram, min_len;
 } case_tail_args_t;
 int case_row_tail(const case_tail_args_t* a, case_stream_t stream);
 int case_row_tail_max_vocab(void);
@@ -606,6 +617,12 @@ typedef struct {
    * not take it (CASE_OPT_DENSE_TAIL / CASE_OPT_UNFUSED_TAIL, materialize_only, no base_* buffers, V < 2W, more than
    * case_sparse_tail_max_sources() source positions) is refused before the first launch. */
   case_attr_t* attr_cand; case_attr_t* attr_hist; case_attr_t* out_attr;
+  /* search constraints (case_tail_args_t.no_repeat_ngram / min_len; 0 = off), modes CASE_MODE_BEAM and
+   * CASE_MODE_PROTO_GREEDY: 0 <= no_repeat_ngram <= max_len, 0 <= min_len < max_len.  The ids compared are the returned
+   * ones (tok_ext with n_oov > 0; greedy: the emitted token).  Only the sparse tail applies them: a request on a step that
+   * would not take it (as for attribution), in CASE_MODE_MODULE_GREEDY, or with V < 2W + Tmax + 1 is refused before the
+   * first launch; the n-best and attribution refusals come first. */
+  int32_t no_repeat_ngram, min_len;
 } case_step_args_t;
 
 /* Enqueue one full decode step t (embedding .. select) for all R rows: the body of the eval loop
@@ -643,6 +660,7 @@ typedef struct {
   /* attribution records (as in case_step_args_t; part[1] = copy from the background, part[2] = 0); refused before the
    * first launch unless the step takes the sparse tail */
   case_attr_t* attr_cand; case_attr_t* attr_hist; case_attr_t* out_attr;
+  int32_t no_repeat_ngram, min_len;                      /* search constraints (as in case_step_args_t) */
 } gttp_step_args_t;
 
 /* One GTTP decode step (GTTP/Model.py:176-193 -> BBCDecoder.forward :113-131 ->
