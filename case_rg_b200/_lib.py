@@ -19,6 +19,16 @@ OPT_NO_PDL, OPT_NO_CHAIN, OPT_NO_STACK, OPT_NO_FORK, OPT_NO_POST, OPT_NO_GATE = 
 OPT_NO_EVICT_FIRST, OPT_DENSE_TAIL, OPT_UNFUSED_TAIL, OPT_NO_FUSED_SELECT, OPT_NO_COPY_PLAN = 0x40, 0x80, 0x100, 0x200, 0x400
 
 vp, i32, f32p = C.c_void_p, C.c_int32, C.c_void_p
+MAX_BAN_SEQ, MAX_BAN_LEN = 256, 16     # CASE_MAX_BAN_SEQ / CASE_MAX_BAN_LEN: banned sequences (length >= 2), their length
+
+
+def _pad(block, full_type):
+    """Give an argument block built as an earlier (shorter) form the storage of the complete one, zeroed: the launchers
+    read every block as the complete struct."""
+    size, full = C.sizeof(type(block)), C.sizeof(full_type)
+    if size < full:
+        C.resize(block, full)
+        C.memset(C.addressof(block) + size, 0, full - size)
 
 
 class Seg(C.Structure):
@@ -78,22 +88,34 @@ class TailArgs(C.Structure):
 
     def __init__(self, *args, **kw):
         # the launchers read every block as the complete case_tail_args_t: a block built as TailArgs gets the storage of
-        # the trailing constraint fields too (zero: no constraints)
+        # the trailing constraint and ban fields too (zero: no constraints, no bans)
         super().__init__(*args, **kw)
-        size, full = C.sizeof(type(self)), C.sizeof(TailConstrArgs)
-        if size < full:
-            C.resize(self, full)
-            C.memset(C.addressof(self) + size, 0, full - size)
+        _pad(self, TailBanArgs)
 
 
 # The search constraints trail the argument blocks (ABI version 2 unchanged), appended by subclassing like the attribution
-# pointers: TailConstrArgs / StepConstrArgs / GttpStepConstrArgs are the complete blocks the launchers read.
+# pointers: TailConstrArgs / StepConstrArgs / GttpStepConstrArgs.
 class TailConstrArgs(TailArgs):
     _fields_ = [('hist_tok', vp), ('hist_anc', vp)] + \
                [(n, i32) for n in ('hist_ld', 't', 'eos', 'no_repeat_ngram', 'min_len')]
 
 
+# The banned words trail them in turn: TailBanArgs / StepBanArgs / GttpStepBanArgs are the complete blocks the launchers
+# read.  ban_mask uint32 [ceil(V / 32)], ban_tok int32 [MAX_BAN_SEQ][MAX_BAN_LEN], ban_len int32 [MAX_BAN_SEQ], ban_n
+# int32 [1], all in device memory (NULL = no bans).
+_BAN_FIELDS = [('ban_mask', vp), ('ban_tok', vp), ('ban_len', vp), ('ban_n', vp)]
+
+
+class TailBanArgs(TailConstrArgs):
+    _fields_ = _BAN_FIELDS
+
+
 class StepArgs(C.Structure):
+    def __init__(self, *args, **kw):
+        # as TailArgs: the storage of every trailing field, zeroed (no attribution, constraints or bans)
+        super().__init__(*args, **kw)
+        _pad(self, StepBanArgs)
+
     _fields_ = [(n, i32) for n in ('B', 'W', 'R', 'V', 'ldv', 'Tmax', 'dtype', 'fast_tanh', 'vocab_impl', 'mode')] + \
                [('S', i32 * 2), ('nsplit_x', i32 * 2), ('nsplit_a', i32 * 2), ('map_off', i32 * 2)] + \
                [(n, i32) for n in ('max_len', 'BOS', 'EOS', 'UNK', 'PAD', 'materialize_only')] + \
@@ -117,7 +139,15 @@ class StepConstrArgs(StepAttrArgs):
     _fields_ = [('no_repeat_ngram', i32), ('min_len', i32)]
 
 
+class StepBanArgs(StepConstrArgs):
+    _fields_ = _BAN_FIELDS
+
+
 class GttpStepArgs(C.Structure):
+    def __init__(self, *args, **kw):
+        super().__init__(*args, **kw)
+        _pad(self, GttpStepBanArgs)
+
     _fields_ = [(n, i32) for n in ('B', 'W', 'R', 'V', 'ldv', 'dtype', 'fast_tanh', 'vocab_impl', 'mode', 'Lc', 'Lb',
                                    'nsplit_c', 'nsplit_b', 'max_len', 'BOS', 'EOS', 'UNK', 'PAD',
                                    'materialize_only', 'Tmax')] + \
@@ -138,6 +168,10 @@ class GttpStepAttrArgs(GttpStepArgs):
 
 class GttpStepConstrArgs(GttpStepAttrArgs):
     _fields_ = [('no_repeat_ngram', i32), ('min_len', i32)]
+
+
+class GttpStepBanArgs(GttpStepConstrArgs):
+    _fields_ = _BAN_FIELDS
 
 
 # name -> argtypes (return type is int for all but the three listed below)
@@ -199,7 +233,7 @@ _PROTOS = {
 _SIZE_FNS = ['case_vocab_tc_workspace_bytes', 'case_vocab_tc_packed_weight_bytes']
 _SIZE_FNS2 = ['case_interaction_smem_bytes', 'case_gemm_rows_packed_weight_bytes']      # (int, int) -> size_t
 EXPORTS = sorted(list(_PROTOS) + ['case_abi_version', 'case_last_error', 'case_struct_size'] + _SIZE_FNS + _SIZE_FNS2)
-_STRUCTS = [Seg, RowLinArgs, LayerWeights, SelectAttrArgs, StepConstrArgs, GttpStepConstrArgs, TailConstrArgs, ChainPost]
+_STRUCTS = [Seg, RowLinArgs, LayerWeights, SelectAttrArgs, StepBanArgs, GttpStepBanArgs, TailBanArgs, ChainPost]
 
 _lib = None
 

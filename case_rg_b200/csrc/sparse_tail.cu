@@ -159,16 +159,25 @@ __device__ __forceinline__ int sp_find(const int* hkeys, int nent, bool plan, in
   }
 }
 
-// Constrained launches (case_tail_args_t.no_repeat_ngram / min_len) append these int arrays to the dynamic shared memory,
-// after the table: the row's answer so far, the ban candidates, the banned ids (one entry per candidate, -1 = none or a
-// repeat of an earlier candidate) and the row's base entries
-constexpr int CS_HIST = 0, CS_CAND = CS_HIST + CASE_MAX_T, CS_BAN = CS_CAND + CASE_MAX_T + 1,
-              CS_BASE = CS_BAN + CASE_MAX_T + 1, CS_INTS = CS_BASE + 2 * SP_PARTS * 2 * CASE_MAX_W;
+// Constrained launches (case_tail_args_t.no_repeat_ngram / min_len / ban_*) append these int arrays to the dynamic shared
+// memory, after the table: the row's answer so far, the ban candidates (t n-gram continuations, the EOS of min_len, one
+// per banned sequence; -1 = none), the banned ids (the distinct candidates, compacted), the row's base entries and the
+// length of the banned list
+constexpr int CS_NCAND = CASE_MAX_T + 1 + CASE_MAX_BAN_SEQ;
+constexpr int CS_HIST = 0, CS_CAND = CS_HIST + CASE_MAX_T, CS_BAN = CS_CAND + CS_NCAND, CS_BASE = CS_BAN + CS_NCAND,
+              CS_NBAN = CS_BASE + 2 * SP_PARTS * 2 * CASE_MAX_W, CS_INTS = CS_NBAN + 1;
+static_assert(CS_NCAND <= TS, "one ban candidate per thread");
 
 __device__ __forceinline__ bool sp_banned(const int* ban, int nban, int id) {
   bool hit = false;
   for (int i = 0; i < nban; ++i) hit |= ban[i] == id;
   return hit;
+}
+
+// single-id bans (case_tail_args_t.ban_mask, NULL = none): bit id of the mask, read through L1 (the few words a row
+// tests are shared by every row of the step, so they stay cached; no shared-memory staging per CTA)
+__device__ __forceinline__ bool sp_masked(const uint32_t* mask, int id, int V) {
+  return mask != nullptr && (unsigned)id < (unsigned)V && ((__ldg(mask + (id >> 5)) >> (id & 31)) & 1u);
 }
 
 // ATTR (case_tail_args_t.attr != NULL): after the top-k, an attribution pass writes the record of every winner (see
@@ -178,7 +187,9 @@ __device__ __forceinline__ bool sp_banned(const int* ban, int nban, int id) {
 // through the base entries only, and the unconstrained argument needs 2K of them (K for the result, K of slack for the
 // ties of the gate scale's rounding).  A banned base entry uses up one of them, so with a = the allowed ids among the
 // row's global top-k2 base entries the row keeps the usual path while a >= 2K and otherwise takes an exact pass over
-// all V logits (offering every allowed untouched id; fbcount counts these rows).
+// all V logits (offering every allowed untouched id; fbcount counts these rows).  Banned words (ban_*) run in the same
+// instance: a banned sequence whose first L - 1 tokens end the answer adds its last token to the banned list, and the
+// single-id mask is tested wherever the list is (touched ids, base entries, the exact pass).
 template <bool ATTR, bool CONSTR>
 __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t a, const float* __restrict__ base_ms,
                                                          const float* __restrict__ base_e,
@@ -225,6 +236,7 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
   // previous step's select wrote it)
   int* const cs = hkeys + (plan ? 2 : 3) * nslots;
   if constexpr (CONSTR) {
+    if (tid == 0) cs[CS_NBAN] = 0;
     for (int j = tid; j < a.t; j += TS) {
       const int p = j + 1;
       const int src = p == a.t ? r : a.hist_anc[(size_t)r * a.hist_ld + p];
@@ -357,9 +369,13 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
   if constexpr (CONSTR) {
     // (both branches above end with a barrier: the history is visible.)  Candidate j < t: the n-gram y_{j+1} ..
     // y_{j+n} lies in the answer and its first n - 1 tokens are the answer's last n - 1, so y_{j+n} is banned;
-    // candidate t: the EOS of an answer shorter than min_len.  An id is kept at its first candidate only
+    // candidate t: the EOS of an answer shorter than min_len; candidate t + 1 + i: banned sequence i = (w_1 .. w_L)
+    // bans w_L when the answer ends with w_1 .. w_{L-1}.  An id is kept at its first candidate only, and the kept ids
+    // are compacted into the banned list (its order does not matter)
     const int t = a.t, n = a.no_repeat_ngram;
-    if (tid <= t) {
+    const int nseq = a.ban_n != nullptr ? min(max(*a.ban_n, 0), CASE_MAX_BAN_SEQ) : 0;
+    const int ncand = t + 1 + nseq;
+    if (tid < ncand) {
       int c = -1;
       if (tid < t) {
         if (n > 0 && tid + n <= t) {
@@ -367,17 +383,26 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
           for (int k = 0; k < n - 1; ++k) eq &= cs[CS_HIST + tid + k] == cs[CS_HIST + t - n + 1 + k];
           if (eq) c = cs[CS_HIST + tid + n - 1];
         }
-      } else if (t < a.min_len) {
-        c = a.eos;
+      } else if (tid == t) {
+        if (t < a.min_len) c = a.eos;
+      } else {
+        const int i = tid - t - 1, L = a.ban_len[i];
+        const int32_t* w = a.ban_tok + (size_t)i * CASE_MAX_BAN_LEN;
+        if (L >= 2 && L <= CASE_MAX_BAN_LEN && t >= L - 1) {
+          bool eq = true;
+          for (int k = 0; k < L - 1; ++k) eq &= cs[CS_HIST + t - L + 1 + k] == w[k];
+          if (eq) c = w[L - 1];
+        }
       }
       cs[CS_CAND + tid] = c;
     }
     __syncthreads();
-    if (tid <= t) {
+    if (tid < ncand) {
       const int c = cs[CS_CAND + tid];
       bool first = c >= 0;
-      for (int j = 0; j < tid; ++j) first &= cs[CS_CAND + j] != c;
-      cs[CS_BAN + tid] = first ? c : -1;
+      if (first)
+        for (int j = 0; j < tid; ++j) first &= cs[CS_CAND + j] != c;
+      if (first) cs[CS_BAN + atomicAdd(cs + CS_NBAN, 1)] = c;
     }
     // (visible after the barrier that ends the copy-mass pass)
   }
@@ -527,19 +552,26 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
     }
   }
   stamp();
-  const int nban = a.t + 1;                              // constrained: entries of the banned list
+  const int nban = CONSTR ? cs[CS_NBAN] : 0;             // constrained: entries of the banned list
+  // constrained: is id banned (the row's list or the single-id mask)?
+  auto banned = [&](int id) { return sp_banned(cs + CS_BAN, nban, id) || sp_masked(a.ban_mask, id, V); };
   if constexpr (CONSTR) {
-    // banned touched ids: one lookup each, the value becomes -inf; then the thread maxima again without them
+    // banned touched ids: one lookup each, the value becomes -inf; then the thread maxima again without them, every
+    // touched id tested against the mask on the way
     __syncthreads();
     if (tid < nban) {
       const int id = cs[CS_BAN + tid];
-      const int sl = id >= 0 ? sp_find(hkeys, nent, plan, id, hshift, hmask) : -1;
+      const int sl = sp_find(hkeys, nent, plan, id, hshift, hmask);
       if (sl >= 0) hvals[sl] = -INFINITY;
     }
     __syncthreads();
     tmax = -INFINITY;
-    for (int sl = tid; sl < nent; sl += TS)
-      if (hkeys[sl] >= 0) tmax = fmaxf(tmax, hvals[sl]);
+    for (int sl = tid; sl < nent; sl += TS) {
+      const int id = hkeys[sl];
+      if (id < 0) continue;
+      if (sp_masked(a.ban_mask, id, V)) hvals[sl] = -INFINITY;
+      else tmax = fmaxf(tmax, hvals[sl]);
+    }
   }
   float fb = -INFINITY;                                  // base candidates that received no copy mass
   int idb = 0x7fffffff;
@@ -565,7 +597,7 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
           slot = (slot + step) & hmask;
         }
       }
-      if (!found && !(CONSTR && sp_banned(cs + CS_BAN, nban, id))) { fb = scl * sp_exp(l - mm); idb = id; }
+      if (!found && !(CONSTR && banned(id))) { fb = scl * sp_exp(l - mm); idb = id; }
     }
   }
   bool exact = false;
@@ -587,7 +619,7 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
     if (tid < SP_PARTS * k2 && l > -INFINITY) {
       int rank = 0;
       for (int j = 0; j < SP_PARTS * k2; ++j) rank += tk_better(bl[j], bi[j], l, id);
-      allowed = rank < k2 && !sp_banned(cs + CS_BAN, nban, id);
+      allowed = rank < k2 && !banned(id);
     }
     exact = __syncthreads_count(allowed) < 2 * K;
   }
@@ -607,7 +639,7 @@ __global__ __launch_bounds__(TS) void sparse_tail_kernel(const case_tail_args_t 
       const int id = v0 + tid;
       float f = -INFINITY;
       if (id < V && !(a.mask_col0 && id == 0) && sp_find(hkeys, nent, plan, id, hshift, hmask) < 0 &&
-          !sp_banned(cs + CS_BAN, nban, id)) {
+          !banned(id)) {
         const float l = x[id];
         if (l > -INFINITY) f = scl * sp_exp(l - mm);
       }
@@ -793,7 +825,9 @@ extern "C" int case_sparse_tail(const case_tail_args_t* a, const float* base_ms,
     CB_REQUIRE((sel->out_attr != nullptr) == (a->attr != nullptr) && (sel->attr_cand == nullptr || sel->attr_cand == a->attr),
                "case_sparse_tail: a fused select with attribution needs attr_cand == the tail's attr (both on or both off)");
   }
-  const bool constr = a->no_repeat_ngram != 0 || a->min_len != 0;
+  const int nbanp = (a->ban_mask != nullptr) + (a->ban_tok != nullptr) + (a->ban_len != nullptr) + (a->ban_n != nullptr);
+  CB_REQUIRE(nbanp == 0 || nbanp == 4, "case_sparse_tail: banned words need all of ban_mask / ban_tok / ban_len / ban_n (or none)");
+  const bool constr = a->no_repeat_ngram != 0 || a->min_len != 0 || nbanp == 4;
   if (constr) {
     CB_REQUIRE(a->no_repeat_ngram >= 0 && a->no_repeat_ngram <= CASE_MAX_T && a->min_len >= 0 && a->min_len < CASE_MAX_T,
                "case_sparse_tail: no_repeat_ngram must be 0..CASE_MAX_T and min_len 0..CASE_MAX_T-1");

@@ -168,12 +168,40 @@ static int check_step_constr(int n, int min_len, int mode, int max_len, int V, i
   return CASE_EINVAL;
 }
 
-// the tail's view of the search state: row r's answer tokens along anc_in (the returned ids: tok_ext when present)
+// Banned words of a step (ban_mask / ban_tok / ban_len / ban_n of the step blocks; all four or none, NULL = off): in a
+// search mode that has them and only where the step takes the sparse tail, like the constraints.  The list itself lives
+// in device memory and the launchers never synchronise, so only the pointers are checked here (the kernel bounds what it
+// reads of the content).  Checked before the first launch of the step, after the constraint check.
+static int check_step_bans(const void* mask, const void* tok, const void* len, const void* n, int mode, int V, int W,
+                           int Tmax, bool sparse, const char* what) {
+  const int set = (mask != nullptr) + (tok != nullptr) + (len != nullptr) + (n != nullptr);
+  if (set == 0) return 0;
+  char msg[256];
+  const char* why = nullptr;
+  if (set != 4)
+    why = "banned words need all of ban_mask / ban_tok / ban_len / ban_n (or none)";
+  else if (mode != CASE_MODE_BEAM && mode != CASE_MODE_PROTO_GREEDY)
+    why = "banned words need CASE_MODE_BEAM or CASE_MODE_PROTO_GREEDY";
+  else if (!sparse)
+    why = "banned words need the sparse tail (not with CASE_OPT_DENSE_TAIL / UNFUSED_TAIL, materialize_only, missing "
+          "base_* buffers, V < 2W or too many source positions)";
+  else if (V < 2 * W + Tmax + 1)
+    why = "banned words need V >= 2W + Tmax + 1";
+  if (why == nullptr) return 0;
+  snprintf(msg, sizeof(msg), "%s: %s", what, why);
+  set_error(msg);
+  return CASE_EINVAL;
+}
+
+// the tail's view of the search state: row r's answer tokens along anc_in (the returned ids: tok_ext when present);
+// needed by the constraints and the banned words alike
 static void set_tail_constr(case_tail_args_t& ta, const int32_t* tok, const int32_t* anc_in, int TL, int t, int EOS,
-                            int n, int min_len) {
-  if (n == 0 && min_len == 0) return;
+                            int n, int min_len, const uint32_t* ban_mask, const int32_t* ban_tok, const int32_t* ban_len,
+                            const int32_t* ban_n) {
+  if (n == 0 && min_len == 0 && ban_mask == nullptr) return;
   ta.hist_tok = tok; ta.hist_anc = anc_in; ta.hist_ld = TL; ta.t = t; ta.eos = EOS;
   ta.no_repeat_ngram = n; ta.min_len = min_len;
+  ta.ban_mask = ban_mask; ta.ban_tok = ban_tok; ta.ban_len = ban_len; ta.ban_n = ban_n;
 }
 
 static void set_select_attr(case_select_args_t& s, case_attr_t* cand, case_attr_t* hist, case_attr_t* out) {
@@ -209,9 +237,10 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
                       a->S[0] + a->S[1] <= case_sparse_tail_max_sources();
   TRY(check_step_attr(a->attr_cand, a->attr_hist, a->out_attr, sparse, "case_decode_step"));
   TRY(check_step_constr(a->no_repeat_ngram, a->min_len, a->mode, a->max_len, a->V, W, a->Tmax, sparse, "case_decode_step"));
+  TRY(check_step_bans(a->ban_mask, a->ban_tok, a->ban_len, a->ban_n, a->mode, a->V, W, a->Tmax, sparse, "case_decode_step"));
   const bool attr = a->out_attr != nullptr;
   // constrained steps ask vocab_base for the most base entries the buffers hold (see sparse_tail.cu: exactness)
-  const int k2b = (a->no_repeat_ngram || a->min_len) ? 2 * CASE_MAX_W : k2;
+  const int k2b = (a->no_repeat_ngram || a->min_len || a->ban_mask) ? 2 * CASE_MAX_W : k2;
   // gate form of the additive attentions: the contexts only feed the mixture gate, so 3 gate-projected numbers
   // per key replace the value rows (needs the sparse tail, which merges gate partials instead of contexts)
   const bool gate = !(opt & CASE_OPT_NO_GATE) && sparse && dt == CASE_BF16 && a->Gv[0] != nullptr && a->Gv[1] != nullptr;
@@ -414,7 +443,8 @@ extern "C" int case_decode_step(const case_step_args_t* a, int t, case_stream_t 
                                            a->ended, a->best_key, a->best_len, a->out_tokens, a->n_live, a->nbest);
       if (n_oov) { sel.V_in = a->V; sel.tok_ext = a->tok_ext; }
       set_select_attr(sel, a->attr_cand, a->attr_hist, a->out_attr);
-      set_tail_constr(ta, n_oov ? a->tok_ext : a->tok, anc, TL, t, a->EOS, a->no_repeat_ngram, a->min_len);
+      set_tail_constr(ta, n_oov ? a->tok_ext : a->tok, anc, TL, t, a->EOS, a->no_repeat_ngram, a->min_len, a->ban_mask,
+                      a->ban_tok, a->ban_len, a->ban_n);
       TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2b, fuse_sel ? &sel : nullptr, a->qcount, st));
       if (fuse_sel) return 0;
     } else {
@@ -473,7 +503,8 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
                       a->V >= k2 && a->Lb <= case_sparse_tail_max_sources();
   TRY(check_step_attr(a->attr_cand, a->attr_hist, a->out_attr, sparse, "gttp_decode_step"));
   TRY(check_step_constr(a->no_repeat_ngram, a->min_len, a->mode, a->max_len, a->V, W, a->Tmax, sparse, "gttp_decode_step"));
-  const int k2b = (a->no_repeat_ngram || a->min_len) ? 2 * CASE_MAX_W : k2;   // as in case_decode_step
+  TRY(check_step_bans(a->ban_mask, a->ban_tok, a->ban_len, a->ban_n, a->mode, a->V, W, a->Tmax, sparse, "gttp_decode_step"));
+  const int k2b = (a->no_repeat_ngram || a->min_len || a->ban_mask) ? 2 * CASE_MAX_W : k2;   // as in case_decode_step
 
   TRY(case_embed_rows(a->E, nullptr, a->tok, TL, t, 1.0f, a->emb, R, st));
   // two additive attentions with the previous GRU state as query (GTTP/Model.py:117-122)
@@ -549,7 +580,8 @@ extern "C" int gttp_decode_step(const gttp_step_args_t* a, int t, case_stream_t 
     ta.S[0] = a->Lb; ta.attn_un[0] = a->attn_un[1];
     ta.top_vals = a->top_vals; ta.top_idx = a->top_idx;
     ta.attr = a->attr_cand;
-    set_tail_constr(ta, a->tok, a->anc[t & 1], TL, t, a->EOS, a->no_repeat_ngram, a->min_len);
+    set_tail_constr(ta, a->tok, a->anc[t & 1], TL, t, a->EOS, a->no_repeat_ngram, a->min_len, a->ban_mask, a->ban_tok,
+                    a->ban_len, a->ban_n);
     TRY(case_sparse_tail(&ta, a->base_ms, a->base_e, a->base_i, k2b, nullptr, nullptr, st));
   } else if (use_tail && a->V <= case_row_tail_max_vocab()) {
     case_tail_args_t ta;

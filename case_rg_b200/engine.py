@@ -13,9 +13,11 @@ Generations.greedy/beam (common/Generations.py:66-190) and the GTTP step (GTTP/M
 """
 import ctypes as C
 import math
+import operator
 import os
-from typing import Dict, NamedTuple, Optional
+from typing import Dict, NamedTuple, Optional, Tuple
 
+import numpy as np
 import torch
 
 from . import _lib as L
@@ -386,6 +388,130 @@ def check_constraints(opt: int, V: int, W: int, nsources: int, Tmax: int, no_rep
                          f'{L.load().case_sparse_tail_max_sources()}')
 
 
+class BadWords(NamedTuple):
+    """A checked ban list (see check_bad_words): the distinct single ids (ascending) and the distinct sequences of two or
+    more ids (in the caller's order)."""
+    singles: Tuple[int, ...]
+    seqs: Tuple[Tuple[int, ...], ...]
+
+
+def _ban_ids(seq) -> Tuple[int, ...]:
+    if isinstance(seq, torch.Tensor):
+        if seq.dim() != 1 or seq.dtype.is_floating_point or seq.dtype.is_complex or seq.dtype == torch.bool:
+            raise ValueError(f'a banned sequence must be a 1-D integer tensor or a list of ints, got {seq.dtype} '
+                             f'{tuple(seq.shape)}')
+        return tuple(seq.tolist())
+    if isinstance(seq, (str, bytes)) or not hasattr(seq, '__iter__'):
+        raise ValueError(f'a banned sequence must be a 1-D integer tensor or a list of ints, got {seq!r}')
+    ids = tuple(seq)
+    if all(type(v) is int for v in ids):                 # the common case, without the per-id checks below
+        return ids
+    for v in ids:
+        if isinstance(v, bool) or not hasattr(v, '__index__'):
+            raise ValueError(f'banned ids must be ints, got {v!r}')
+    return tuple(operator.index(v) for v in ids)
+
+
+def _check_bans_servable(opt: int, V: int, W: int, nsources: int, Tmax: int, mode: Optional[int] = None) -> None:
+    """Bans run in the sparse tail's constrained instance: ValueError where a search cannot take it."""
+    if mode is not None and mode not in (L.MODE_BEAM, L.MODE_PROTO_GREEDY):
+        raise ValueError('bad_words apply to the beam and greedy searches (not module_greedy)')
+    if opt & (L.OPT_DENSE_TAIL | L.OPT_UNFUSED_TAIL):
+        raise ValueError('bad_words need the sparse tail: not with OPT_DENSE_TAIL / OPT_UNFUSED_TAIL')
+    if nsources > L.load().case_sparse_tail_max_sources():
+        raise ValueError(f'bad_words need the sparse tail: {nsources} source positions exceed its '
+                         f'{L.load().case_sparse_tail_max_sources()}')
+    if V < 2 * W + Tmax + 1:
+        raise ValueError(f'bad_words need V >= 2 * width + max_target_length + 1 (V = {V}, width = {W}, '
+                         f'max_target_length = {Tmax})')
+
+
+def check_bad_words(opt: int, V: int, W: int, nsources: int, Tmax: int, bad_words,
+                    mode: Optional[int] = None) -> Optional[BadWords]:
+    """Banned words (a list of token-id sequences, each a list of ints or a 1-D integer tensor; None or empty = off) ->
+    the checked BadWords, or None when off.  ValueError for a list or a search the device cannot serve: ids outside
+    [0, V) (dynamic OOV ids differ per query), an empty sequence, more than MAX_BAN_SEQ sequences of two or more ids, a
+    sequence longer than MAX_BAN_LEN, no sparse tail (OPT_DENSE_TAIL / OPT_UNFUSED_TAIL, too many source positions),
+    module_greedy (mode), or fewer than 2 * width + max_target_length + 1 + (sequences) ids left allowed.  Duplicates are
+    dropped; a BadWords is checked against the search only."""
+    if bad_words is None:
+        return None
+    if isinstance(bad_words, torch.Tensor) or isinstance(bad_words, (str, bytes)):
+        raise ValueError('bad_words must be a list of token-id sequences (lists of ints or 1-D integer tensors)')
+    if isinstance(bad_words, BadWords):                   # checked already: only the search-dependent limits
+        singles, seqs = bad_words.singles, bad_words.seqs
+        if not 0 <= len(seqs) <= L.MAX_BAN_SEQ or (singles and not 0 <= min(singles) <= max(singles) < V):
+            raise ValueError('bad_words: a BadWords outside the limits')
+        return _check_ban_counts(opt, V, W, nsources, Tmax, bad_words, mode)
+    singles, seqs = set(), {}                             # seqs: an insertion-ordered set
+    for seq in bad_words:
+        ids = _ban_ids(seq)
+        if not ids:
+            raise ValueError('bad_words: a banned sequence is empty')
+        if len(ids) > L.MAX_BAN_LEN:
+            raise ValueError(f'bad_words: a sequence of {len(ids)} ids exceeds MAX_BAN_LEN = {L.MAX_BAN_LEN}')
+        if not (0 <= min(ids) and max(ids) < V):
+            bad = next(v for v in ids if not 0 <= v < V)
+            raise ValueError(f'bad_words: id {bad} outside [0, V = {V}) (dynamic OOV ids cannot be banned by value)')
+        if len(ids) == 1:
+            singles.add(ids[0])
+        else:
+            seqs[ids] = None
+    if not singles and not seqs:
+        return None
+    if len(seqs) > L.MAX_BAN_SEQ:
+        raise ValueError(f'bad_words: {len(seqs)} sequences of two or more ids exceed MAX_BAN_SEQ = {L.MAX_BAN_SEQ}')
+    return _check_ban_counts(opt, V, W, nsources, Tmax, BadWords(tuple(sorted(singles)), tuple(seqs)), mode)
+
+
+def _check_ban_counts(opt, V, W, nsources, Tmax, bw: BadWords, mode) -> Optional[BadWords]:
+    if not bw.singles and not bw.seqs:
+        return None
+    _check_bans_servable(opt, V, W, nsources, Tmax, mode)
+    if V - len(bw.singles) < 2 * W + Tmax + 1 + len(bw.seqs):
+        raise ValueError(f'bad_words leave too few ids: need V - (single ids) >= 2 * width + max_target_length + 1 + '
+                         f'(sequences) (V = {V}, {len(bw.singles)} single ids, width = {W}, max_target_length = {Tmax}, '
+                         f'{len(bw.seqs)} sequences)')
+    return bw
+
+
+class _BanBuffers:
+    """Fixed-capacity device copy of a ban list, the layout of case_tail_args_t.ban_*: one int32 buffer holding the
+    single-id bit mask [ceil(V / 32)], the sequence table [MAX_BAN_SEQ][MAX_BAN_LEN], the lengths [MAX_BAN_SEQ] and the
+    count.  ``write`` replaces the content with a stream-ordered copy on the current stream, so a decode (or a captured
+    graph) enqueued after it reads the new list and the ones enqueued before it read the old one."""
+
+    def __init__(self, dev, V):
+        self.nw = (V + 31) // 32
+        nt = L.MAX_BAN_SEQ * L.MAX_BAN_LEN
+        self.buf = torch.zeros(self.nw + nt + L.MAX_BAN_SEQ + 1, dtype=torch.int32, device=dev)
+        self.mask = self.buf[:self.nw]
+        self.tok = self.buf[self.nw:self.nw + nt]
+        self.len = self.buf[self.nw + nt:self.nw + nt + L.MAX_BAN_SEQ]
+        self.n = self.buf[self.nw + nt + L.MAX_BAN_SEQ:]
+        self.current = BadWords((), ())                      # what the buffer holds (the zeros: nothing banned)
+
+    def bind(self, a):
+        a.ban_mask, a.ban_tok, a.ban_len, a.ban_n = (self.mask.data_ptr(), self.tok.data_ptr(), self.len.data_ptr(),
+                                                     self.n.data_ptr())
+
+    def write(self, bw: BadWords):
+        if bw == self.current:
+            return
+        nt = L.MAX_BAN_SEQ * L.MAX_BAN_LEN
+        host = np.zeros(self.buf.numel(), dtype=np.uint32)
+        ids = np.asarray(bw.singles, dtype=np.int64)
+        np.bitwise_or.at(host, ids >> 5, (np.ones_like(ids) << (ids & 31)).astype(np.uint32))
+        for i, seq in enumerate(bw.seqs):
+            host[self.nw + i * L.MAX_BAN_LEN:self.nw + i * L.MAX_BAN_LEN + len(seq)] = seq
+            host[self.nw + nt + i] = len(seq)
+        host[-1] = len(bw.seqs)
+        # pinned: the copy is asynchronous on the current stream; the caching host allocator keeps the block until it
+        # has been read
+        self.buf.copy_(torch.from_numpy(host.view(np.int32)).pin_memory(), non_blocking=True)
+        self.current = bw
+
+
 class _SearchState:
     """Buffers shared by both engines for the on-device greedy / beam bookkeeping.  nbest > 1: the beam search keeps
     the nbest best finished hypotheses of every query (best_key / best_len [B, nbest], out_tokens [B, nbest, Tmax]).
@@ -469,6 +595,19 @@ class _EngineBase:
         n, m = self.constraints
         if n or m:
             check_constraints(int(self.args.opt), self.V, self.W, 0, self.Tmax, n, m, max_len, mode)
+        if self.bans is not None:
+            _check_bans_servable(int(self.args.opt), self.V, self.W, 0, self.Tmax, mode)
+
+    def set_bad_words(self, bad_words) -> None:
+        """The ban list of the decodes launched after this call (an engine built with bans=True; see check_bad_words; a
+        checked BadWords is taken as it is).  None or empty: nothing banned.  The list is copied into the engine's
+        buffers on the current stream - no new graph capture, no host synchronisation."""
+        if self.bans is None:
+            if bad_words:
+                raise ValueError('this engine was built without bans=True')
+            return
+        bw = check_bad_words(int(self.args.opt), self.V, self.W, 0, self.Tmax, bad_words)
+        self.bans.write(bw if bw is not None else BadWords((), ()))
 
     def _step(self, t: int, cuda_stream: int):
         if self.use_torch_ops:
@@ -527,13 +666,14 @@ class CaseDecodeEngine(_EngineBase):
     def __init__(self, weights: CaseWeights, B: int, W: int, S0: int, S1: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
                  opt: int = 0, n_oov: int = 0, nbest: int = 1, attribution: bool = False, no_repeat_ngram: int = 0,
-                 min_len: int = 0):
+                 min_len: int = 0, bans: bool = False):
         """n_oov > 0: extended vocabulary - ``source_map`` entries in [V, V + n_oov) are per-query dynamic (OOV) words,
         the mixture and its top-k range over V + n_oov ids (pointer-generator extension; an OOV id is fed back as UNK).
         nbest (1..W): a beam decode keeps the nbest best finished hypotheses per query (read with ``_finish_nbest``).
         attribution: every decode also records where each answer token came from (read with ``_finish_attribution``).
         no_repeat_ngram / min_len: search constraints of every beam / greedy decode (0 = off; see
-        generations.beam): no answer repeats an n-gram, EOS is banned before step min_len."""
+        generations.beam): no answer repeats an n-gram, EOS is banned before step min_len.
+        bans: the engine owns ban-list buffers and every decode applies the list last given to ``set_bad_words``."""
         self.opt, self.n_oov = int(opt), int(n_oov)
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
@@ -541,6 +681,9 @@ class CaseDecodeEngine(_EngineBase):
             check_attribution(self.opt, weights.V, W, S0 + S1)
         check_constraints(self.opt, weights.V, W, S0 + S1, Tmax, no_repeat_ngram, min_len)
         self.constraints = (int(no_repeat_ngram), int(min_len))
+        if bans:
+            _check_bans_servable(self.opt, weights.V, W, S0 + S1, Tmax)
+        self.bans = _BanBuffers(weights.device, weights.V) if bans else None
         self.nparts = 3
         if not (1 <= Tmax <= L.MAX_T):
             raise ValueError(f'max_target_length must be 1..{L.MAX_T}')
@@ -639,8 +782,10 @@ class CaseDecodeEngine(_EngineBase):
         self._fill_args()
 
     def _fill_args(self):
-        a = self.args = L.StepConstrArgs()
+        a = self.args = L.StepBanArgs()
         a.no_repeat_ngram, a.min_len = self.constraints
+        if self.bans is not None:
+            self.bans.bind(a)
         w = self.w
         a.opt, a.fork = self.opt, self._fork.h
         if self.n_oov:
@@ -798,6 +943,8 @@ class CaseDecodeEngine(_EngineBase):
         [R, V] of it (no top-k / select); the caller drives tok/anc through ``state``."""
         if any(self.constraints):
             raise ValueError('no_repeat_ngram / min_len apply to the beam and greedy searches, not to the `generate` face')
+        if self.bans is not None:
+            raise ValueError('bad_words apply to the beam and greedy searches, not to the `generate` face')
         for i in range(2):
             if self._mv_src[i] is not None:
                 self.Mv[i].copy_(self._mv_src[i].view_as(self.Mv[i]))
@@ -857,13 +1004,17 @@ class GttpWeights:
 class GttpDecodeEngine(_EngineBase):
     def __init__(self, weights: GttpWeights, B: int, W: int, Lc: int, Lb: int, Tmax: int = 40,
                  fast_tanh: Optional[bool] = None, vocab_impl: Optional[int] = None, target_ctas: int = 296,
-                 opt: int = 0, nbest: int = 1, attribution: bool = False, no_repeat_ngram: int = 0, min_len: int = 0):
+                 opt: int = 0, nbest: int = 1, attribution: bool = False, no_repeat_ngram: int = 0, min_len: int = 0,
+                 bans: bool = False):
         if not (1 <= W <= L.MAX_W):
             raise ValueError(f'beam width must be 1..{L.MAX_W}')
         if attribution:
             check_attribution(int(opt), weights.V, W, Lb)
         check_constraints(int(opt), weights.V, W, Lb, Tmax, no_repeat_ngram, min_len)
         self.constraints = (int(no_repeat_ngram), int(min_len))
+        if bans:
+            _check_bans_servable(int(opt), weights.V, W, Lb, Tmax)
+        self.bans = _BanBuffers(weights.device, weights.V) if bans else None
         self.nparts = 2
         self.w = weights
         self.device = dev = weights.device
@@ -903,8 +1054,10 @@ class GttpDecodeEngine(_EngineBase):
         self._graphs = {}
         self._step_fn = L.load().gttp_decode_step
         self._step_name = 'gttp_decode_step'
-        a = self.args = L.GttpStepConstrArgs()
+        a = self.args = L.GttpStepBanArgs()
         a.no_repeat_ngram, a.min_len = self.constraints
+        if self.bans is not None:
+            self.bans.bind(a)
         w = weights
         a.B, a.W, a.R, a.V, a.ldv, a.dtype = B, W, R, V, self.ldv, w.cdtype
         a.opt = int(opt)

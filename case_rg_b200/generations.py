@@ -19,6 +19,15 @@ so every answer has at least m tokens before its EOS.  Banned ids leave the cand
 a chosen token still costs -log(p + 1e-10) under the model's mixture, so costs stay comparable with unconstrained
 searches.  The ids compared are the returned ones (extended-vocabulary ids; greedy: the emitted token).
 
+Every search face also takes ``bad_words``: a list of token-id sequences (lists of ints or 1-D integer tensors) that no
+answer may contain.  A single id is never a candidate; a sequence (w_1 .. w_L) bans w_L wherever the answer so far ends
+with w_1 .. w_{L-1}, so no answer and no n-best entry contains it contiguously.  The same rule as the constraints:
+nothing is renormalised, costs stay those of the model's mixture.  Unlike GTTP's fixed mask of id 0 (removed from the
+softmax itself), a banned id keeps its share of the distribution.  In ``greedy`` an EOS chosen at t = 0 is still
+rewritten to UNK (Generations.py:99-100), even when UNK is banned; ``min_len >= 1`` prevents that.  None or empty (the
+default) is the unbanned search.  Ids must lie in [0, V); at most 256 sequences of two or more ids, each at most 16
+long (_lib.MAX_BAN_SEQ / MAX_BAN_LEN), and V - (single ids) >= 2 * width + max_len + 1 + (sequences).
+
 ``FastCaSE`` gives the unchanged CaSE decoder the protocol the reference never implemented for it
 (SURVEY.md §8c adapter); ``FastGTTP`` replaces ``GTTP.decode/generate/to_word`` + the search
 (GTTP/Model.py:176-193).  Both take the *encoder-side outputs* as inputs: the encoders are outside
@@ -30,7 +39,7 @@ import torch
 
 from . import _lib as L
 from .engine import (Attributed, CaseDecodeEngine, CaseWeights, GttpDecodeEngine, GttpWeights, NBest, attributed_from,
-                     check_constraints, nbest_from)
+                     check_bad_words, check_constraints, nbest_from)
 
 PAD_WORD, BOS_WORD, UNK_WORD, EOS_WORD = '[PAD]', '[unused0]', '[UNK]', '[unused1]'
 
@@ -45,19 +54,21 @@ def _check_vocab(vocab2id):
 
 
 def greedy(model, data, vocab2id=None, max_len=20, encode_outputs=None, init_decoder_states=None, no_repeat_ngram=0,
-           min_len=0):
-    """Generations.greedy (Generations.py:66-110) on the device; no_repeat_ngram / min_len: see the module docstring."""
+           min_len=0, bad_words=None):
+    """Generations.greedy (Generations.py:66-110) on the device; no_repeat_ngram / min_len / bad_words: see the module
+    docstring."""
     _check_vocab(vocab2id)
     return model.fast_search(data, max_len, 1, L.MODE_PROTO_GREEDY, encode_outputs, init_decoder_states,
-                             no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                             no_repeat_ngram=no_repeat_ngram, min_len=min_len, bad_words=bad_words)
 
 
 def beam(model, data, vocab2id=None, max_len=20, width=5, encode_outputs=None, init_decoder_states=None,
-         no_repeat_ngram=0, min_len=0):
-    """Generations.beam (Generations.py:112-190) on the device; no_repeat_ngram / min_len: see the module docstring."""
+         no_repeat_ngram=0, min_len=0, bad_words=None):
+    """Generations.beam (Generations.py:112-190) on the device; no_repeat_ngram / min_len / bad_words: see the module
+    docstring."""
     _check_vocab(vocab2id)
     return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states,
-                             no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                             no_repeat_ngram=no_repeat_ngram, min_len=min_len, bad_words=bad_words)
 
 
 def _nbest_count(n, width):
@@ -68,64 +79,68 @@ def _nbest_count(n, width):
 
 
 def beam_nbest(model, data, vocab2id=None, max_len=20, width=5, n=None, encode_outputs=None, init_decoder_states=None,
-               no_repeat_ngram=0, min_len=0):
+               no_repeat_ngram=0, min_len=0, bad_words=None):
     """The n best answers of ``beam`` per query with their costs: ``NBest(tokens, lengths, costs)`` on the model's
     device, entry [:, i] the i-th of sorted(results[q], key=cum_cost/length)[:n] (Generations.py:183-185).  tokens int64
     [B, n, L] (BOS dropped, EOS kept, zero padded to the longest entry), lengths int64 [B, n], costs fp64 [B, n] = the
     ranking key cum_cost / length in nats per position (lower is better).  Entry 0 is what ``beam`` returns.  n defaults
-    to the width; 1 <= n <= width.  With no_repeat_ngram / min_len every entry satisfies the constraints."""
+    to the width; 1 <= n <= width.  With no_repeat_ngram / min_len / bad_words every entry satisfies the constraints and
+    contains no banned word."""
     _check_vocab(vocab2id)
     n = _nbest_count(n, width)
     return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states, nbest=n,
-                             no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                             no_repeat_ngram=no_repeat_ngram, min_len=min_len, bad_words=bad_words)
 
 
 def beam_attributed(model, data, vocab2id=None, max_len=20, width=5, n=None, encode_outputs=None,
-                    init_decoder_states=None, no_repeat_ngram=0, min_len=0):
+                    init_decoder_states=None, no_repeat_ngram=0, min_len=0, bad_words=None):
     """``beam_nbest`` with the attribution record of every answer token: ``Attributed(answer, parts, source)`` on the
     model's device, ``answer`` the NBest of ``beam_nbest`` (the same search, bit for bit), ``parts`` fp32 [B, n, L, P] and
     ``source`` int64 [B, n, L], trimmed like the tokens (see engine.Attributed).  n defaults to the width."""
     _check_vocab(vocab2id)
     n = _nbest_count(n, width)
     return model.fast_search(data, max_len, width, L.MODE_BEAM, encode_outputs, init_decoder_states, nbest=n,
-                             attribution=True, no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                             attribution=True, no_repeat_ngram=no_repeat_ngram, min_len=min_len, bad_words=bad_words)
 
 
 def greedy_attributed(model, data, vocab2id=None, max_len=20, encode_outputs=None, init_decoder_states=None,
-                      no_repeat_ngram=0, min_len=0):
+                      no_repeat_ngram=0, min_len=0, bad_words=None):
     """``greedy`` with the attribution record of every answer token: ``Attributed(answer, parts, source)``, ``answer`` the
     LongTensor [B, max_len] of ``greedy``, ``parts`` fp32 [B, max_len, P], ``source`` int64 [B, max_len].  At t = 0 an
     EOS rewritten to UNK keeps the record of the EOS the distribution chose; PAD positions after the end have zero parts
     and source -1."""
     _check_vocab(vocab2id)
     return model.fast_search(data, max_len, 1, L.MODE_PROTO_GREEDY, encode_outputs, init_decoder_states,
-                             attribution=True, no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                             attribution=True, no_repeat_ngram=no_repeat_ngram, min_len=min_len, bad_words=bad_words)
 
 
 def beam_batches(model, batches, vocab2id=None, max_len=20, width=5, n_best=None, attribution=False, no_repeat_ngram=0,
-                 min_len=0):
+                 min_len=0, bad_words=None):
     """``beam`` over an iterable of HOST batches, the way the predict loop feeds a model one batch after
     another (common/CumulativeTrainer.py:141-156): yields the answers of every batch, in order, as host
     LongTensors.  The host-to-device copy of batch i+1 runs on a copy stream while batch i is decoding
     (double-buffered staging, pinned host tensors copy asynchronously), so the PCIe time of the encoder
     outputs (175 MB per batch at the BASELINE shape) is hidden behind the decode.  n_best: yields the ``beam_nbest``
     lists of every batch instead (NBest of host tensors).  attribution: yields what ``beam_attributed(..., n=n_best)``
-    returns for every batch (host Attributed; n_best None = the width).  no_repeat_ngram / min_len: the constraints of
-    ``beam`` (checked here, before the first batch is read)."""
+    returns for every batch (host Attributed; n_best None = the width).  no_repeat_ngram / min_len / bad_words: the
+    constraints and bans of ``beam`` (checked here, before the first batch is read; the ban list is written to the
+    engine once, before the first prefill)."""
     _check_vocab(vocab2id)
     if n_best is not None or attribution:
         n_best = _nbest_count(n_best, width)
-    model._check_constraints(max_len, width, L.MODE_BEAM, no_repeat_ngram, min_len)
-    return model.search_batches(batches, max_len, width, L.MODE_BEAM, n_best, attribution, no_repeat_ngram, min_len)
+    bw = model._check_constraints(max_len, width, L.MODE_BEAM, no_repeat_ngram, min_len, bad_words)
+    return model.search_batches(batches, max_len, width, L.MODE_BEAM, n_best, attribution, no_repeat_ngram, min_len, bw)
 
 
-def greedy_batches(model, batches, vocab2id=None, max_len=20, attribution=False, no_repeat_ngram=0, min_len=0):
+def greedy_batches(model, batches, vocab2id=None, max_len=20, attribution=False, no_repeat_ngram=0, min_len=0,
+                   bad_words=None):
     """``greedy`` over an iterable of host batches with the copy of the next batch overlapped (see beam_batches).
     attribution: yields what ``greedy_attributed`` returns for every batch (host Attributed).  no_repeat_ngram /
-    min_len: the constraints of ``greedy``."""
+    min_len / bad_words: the constraints and bans of ``greedy``."""
     _check_vocab(vocab2id)
-    model._check_constraints(max_len, 1, L.MODE_PROTO_GREEDY, no_repeat_ngram, min_len)
-    return model.search_batches(batches, max_len, 1, L.MODE_PROTO_GREEDY, None, attribution, no_repeat_ngram, min_len)
+    bw = model._check_constraints(max_len, 1, L.MODE_PROTO_GREEDY, no_repeat_ngram, min_len, bad_words)
+    return model.search_batches(batches, max_len, 1, L.MODE_PROTO_GREEDY, None, attribution, no_repeat_ngram, min_len,
+                                bw)
 
 
 def _to_host(att: Attributed) -> Attributed:
@@ -160,13 +175,13 @@ class _FastModel:
 
     # ---- streamed batches (beam_batches / greedy_batches)
     def search_batches(self, batches, max_len, width, mode, n_best=None, attribution=False, no_repeat_ngram=0,
-                       min_len=0):
+                       min_len=0, bad_words=None):
         """Generator behind beam_batches / greedy_batches (n_best: beam mode, yields NBest per batch; attribution: yields
-        Attributed per batch; no_repeat_ngram / min_len: the search constraints)."""
+        Attributed per batch; no_repeat_ngram / min_len / bad_words: the search constraints and bans)."""
         dev = self.weights.device
         if attribution:
             self._check_attribution_opt()
-        self._check_constraints(max_len, width, mode, no_repeat_ngram, min_len)
+        bw = self._check_constraints(max_len, width, mode, no_repeat_ngram, min_len, bad_words)
         main = torch.cuda.current_stream(dev)
         # the copy stream and the two staging sets live as long as the model: allocating 2 x 175 MB on a
         # fresh stream per call costs tens of milliseconds of cudaMalloc
@@ -205,7 +220,7 @@ class _FastModel:
             # decoding is never prefilled: engine_for returns the SAME engine for equal shapes, and its decode is
             # ahead of this prefill on the main stream)
             main.wait_event(ready)
-            eng = self._prefill_staged(d, width, max_len, n_best or 1, attribution, no_repeat_ngram, min_len)
+            eng = self._prefill_staged(d, width, max_len, n_best or 1, attribution, no_repeat_ngram, min_len, bw)
             prefilled[k] = torch.cuda.Event()
             prefilled[k].record(main)
             nxt = next(it, None)
@@ -265,10 +280,12 @@ class _FastModel:
         if self.opt & (L.OPT_DENSE_TAIL | L.OPT_UNFUSED_TAIL):
             raise ValueError('attribution needs the sparse tail: not with OPT_DENSE_TAIL / OPT_UNFUSED_TAIL')
 
-    def _check_constraints(self, max_len, width, mode, no_repeat_ngram, min_len):
-        """no_repeat_ngram / min_len: ValueError for a request the device search cannot serve, before anything is built
-        (the engines of a search are sized Tmax = max_len; the source count is checked when the engine is built)."""
+    def _check_constraints(self, max_len, width, mode, no_repeat_ngram, min_len, bad_words=None):
+        """no_repeat_ngram / min_len / bad_words: ValueError for a request the device search cannot serve, before anything
+        is built (the engines of a search are sized Tmax = max_len; the source count is checked when the engine is
+        built).  -> the checked ban list (engine.BadWords), None when there is none."""
         check_constraints(self.opt, self.weights.V, width, 0, max_len, no_repeat_ngram, min_len, max_len, mode)
+        return check_bad_words(self.opt, self.weights.V, width, 0, max_len, bad_words, mode)
 
     def _finish(self, eng, max_len, mode, nbest, attribution):
         """Answers of the decode just launched on ``eng``: tokens, the NBest list (nbest), or Attributed (attribution)."""
@@ -304,12 +321,13 @@ class FastCaSE(_FastModel):
             self.producers = CaseProducers(producers, device=self.weights.device)
 
     def search_ids(self, data, max_len=None, width=None, mode='beam', n_best=None, attribution=False, no_repeat_ngram=0,
-                   min_len=0):
+                   min_len=0, bad_words=None):
         """CaSE.do_test from token ids (CaSE/Model.py:313-331): ``data`` = {'query' int [B,1,Lq], 'passage' int [B,NP,Lp],
         'source_map' int [B,S]} -> {'answer': LongTensor, 'rank': [B,NP]} like the reference's forward(data, 'test').
         n_best (beam mode): also 'nbest', the ``beam_nbest`` list of the same search (its entry 0 is 'answer').
         attribution (every mode): also 'attribution', the Attributed of the same search - its answer is the NBest with
-        n_best, else 'answer'.  no_repeat_ngram / min_len (beam and greedy modes): the search constraints of ``beam``."""
+        n_best, else 'answer'.  no_repeat_ngram / min_len / bad_words (beam and greedy modes): the search constraints and
+        bans of ``beam``."""
         if self.producers is None:
             raise RuntimeError('FastCaSE was built without producers=...')
         max_len = self.max_dec_len if max_len is None else max_len
@@ -321,12 +339,12 @@ class FastCaSE(_FastModel):
         if attribution:
             self._check_attribution_opt()
         m = {'beam': L.MODE_BEAM, 'greedy': L.MODE_PROTO_GREEDY, 'module_greedy': L.MODE_MODULE_GREEDY}[mode]
-        self._check_constraints(max_len, width, m, no_repeat_ngram, min_len)
+        bw = self._check_constraints(max_len, width, m, no_repeat_ngram, min_len, bad_words)
         p = self.producers(data['query'], data['passage'])
         d = dict(mem_q=p['mem_q'], mem_p=p['mem_p'], query=data['query'].to(self.weights.device),
                  passage=data['passage'].to(self.weights.device), prior_q=p['prior_q'], prior_p=p['prior_p'],
                  answer_rep=p['answer_rep'], source_map=data['source_map'].to(self.weights.device))
-        cons = dict(no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+        cons = dict(no_repeat_ngram=no_repeat_ngram, min_len=min_len, bad_words=bw)
         if n_best is None and not attribution:
             return {'answer': self.fast_search(d, max_len, width, m, **cons), 'rank': p['rank']}
         got = self.fast_search(d, max_len, width, m, nbest=n_best, attribution=attribution, **cons)
@@ -337,33 +355,30 @@ class FastCaSE(_FastModel):
             out['attribution'] = got
         return out
 
-    def engine_for(self, B, W, S0, S1, T, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0):
-        # the constraints are captured in the engine's CUDA graphs: part of the key
-        key = (B, W, S0, S1, T, self.opt, self.n_oov, nbest, bool(attribution), int(no_repeat_ngram), int(min_len))
+    def engine_for(self, B, W, S0, S1, T, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0, bans=False):
+        # the constraints are captured in the engine's CUDA graphs: part of the key.  The ban list is not (an engine built
+        # with bans reads it from its buffers at every launch), only whether there is one
+        key = (B, W, S0, S1, T, self.opt, self.n_oov, nbest, bool(attribution), int(no_repeat_ngram), int(min_len)) + \
+            ((True,) if bans else ())
         if key not in self._engines:
             if len(self._engines) >= 4:
                 self._engines.clear()
             self._engines[key] = CaseDecodeEngine(self.weights, B, W, S0, S1, T, vocab_impl=self.vocab_impl,
                                                   opt=self.opt, n_oov=self.n_oov, nbest=nbest, attribution=attribution,
-                                                  no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                                                  no_repeat_ngram=no_repeat_ngram, min_len=min_len, bans=bans)
         return self._engines[key]
 
     def encode(self, data):
         return data
 
     def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None,
-                    attribution=False, no_repeat_ngram=0, min_len=0):
+                    attribution=False, no_repeat_ngram=0, min_len=0, bad_words=None):
         """-> the answers (LongTensor), with nbest the NBest list of a beam search, with attribution an Attributed."""
         if attribution:
             self._check_attribution_opt()
-        self._check_constraints(max_len, width, mode, no_repeat_ngram, min_len)
+        bw = self._check_constraints(max_len, width, mode, no_repeat_ngram, min_len, bad_words)
         d = encode_outputs if encode_outputs is not None else data
-        B = d['source_map'].size(0)
-        S0 = d['mem_q'].reshape(B, -1, L.H).size(1)
-        S1 = d['mem_p'].reshape(B, -1, L.H).size(1)
-        eng = self.engine_for(B, width, S0, S1, max_len, nbest or 1, attribution, no_repeat_ngram, min_len)
-        eng.prefill(d['mem_q'], d['mem_p'], d['query'].ne(0), d['passage'].ne(0), d['prior_q'], d['prior_p'],
-                    d['answer_rep'], d['source_map'])
+        eng = self._prefill_staged(d, width, max_len, nbest or 1, attribution, no_repeat_ngram, min_len, bw)
         self.last_engine = eng
         if nbest is None and not attribution:
             return eng.decode(max_len, mode, use_graph=self.use_graph)
@@ -374,11 +389,15 @@ class FastCaSE(_FastModel):
 
     _KEYS = ('mem_q', 'mem_p', 'query', 'passage', 'prior_q', 'prior_p', 'answer_rep', 'source_map')
 
-    def _prefill_staged(self, d, width, max_len, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0):
+    def _prefill_staged(self, d, width, max_len, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0,
+                        bad_words=None):
+        """Engine of the batch d, prefilled; bad_words (a checked BadWords or None) is written to its ban buffers first."""
         B = d['source_map'].size(0)
         S0 = d['mem_q'].reshape(B, -1, L.H).size(1)
         S1 = d['mem_p'].reshape(B, -1, L.H).size(1)
-        eng = self.engine_for(B, width, S0, S1, max_len, nbest, attribution, no_repeat_ngram, min_len)
+        eng = self.engine_for(B, width, S0, S1, max_len, nbest, attribution, no_repeat_ngram, min_len,
+                              bad_words is not None)
+        eng.set_bad_words(bad_words)
         eng.prefill(d['mem_q'], d['mem_p'], d['query'].ne(0), d['passage'].ne(0), d['prior_q'], d['prior_p'],
                     d['answer_rep'], d['source_map'])
         return eng
@@ -400,28 +419,28 @@ class FastGTTP(_FastModel):
         self.opt = int(opt)
         self._engines = {}
 
-    def engine_for(self, B, W, Lc, Lb, T, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0):
-        key = (B, W, Lc, Lb, T, nbest, bool(attribution), int(no_repeat_ngram), int(min_len))
+    def engine_for(self, B, W, Lc, Lb, T, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0, bans=False):
+        key = (B, W, Lc, Lb, T, nbest, bool(attribution), int(no_repeat_ngram), int(min_len)) + ((True,) if bans else ())
         if key not in self._engines:
             if len(self._engines) >= 4:
                 self._engines.clear()
             self._engines[key] = GttpDecodeEngine(self.weights, B, W, Lc, Lb, T, vocab_impl=self.vocab_impl,
                                                   opt=self.opt, nbest=nbest, attribution=attribution,
-                                                  no_repeat_ngram=no_repeat_ngram, min_len=min_len)
+                                                  no_repeat_ngram=no_repeat_ngram, min_len=min_len, bans=bans)
         return self._engines[key]
 
     def fast_search(self, data, max_len, width, mode, encode_outputs=None, init_decoder_states=None, nbest=None,
-                    attribution=False, no_repeat_ngram=0, min_len=0):
+                    attribution=False, no_repeat_ngram=0, min_len=0, bad_words=None):
         """-> the answers (LongTensor), with nbest the NBest list of a beam search, with attribution an Attributed."""
         if attribution:
             self._check_attribution_opt()
-        self._check_constraints(max_len, width, mode, no_repeat_ngram, min_len)
+        bw = self._check_constraints(max_len, width, mode, no_repeat_ngram, min_len, bad_words)
         d = dict(data)
         if encode_outputs is not None:
             d.update(encode_outputs)
         if init_decoder_states is not None:
             d['init_state'] = init_decoder_states
-        eng = self._prefill_staged(d, width, max_len, nbest or 1, attribution, no_repeat_ngram, min_len)
+        eng = self._prefill_staged(d, width, max_len, nbest or 1, attribution, no_repeat_ngram, min_len, bw)
         self.last_engine = eng
         if nbest is None and not attribution:
             return eng.decode(max_len, mode, use_graph=self.use_graph)
@@ -430,10 +449,13 @@ class FastGTTP(_FastModel):
 
     _KEYS = ('context', 'background', 'background_map', 'src_output', 'bg_output', 'init_state')
 
-    def _prefill_staged(self, d, width, max_len, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0):
+    def _prefill_staged(self, d, width, max_len, nbest=1, attribution=False, no_repeat_ngram=0, min_len=0,
+                        bad_words=None):
         B, Lc = d['context'].shape
         Lb = d['background'].size(1)
-        eng = self.engine_for(B, width, Lc, Lb, max_len, nbest, attribution, no_repeat_ngram, min_len)
+        eng = self.engine_for(B, width, Lc, Lb, max_len, nbest, attribution, no_repeat_ngram, min_len,
+                              bad_words is not None)
+        eng.set_bad_words(bad_words)
         eng.prefill(d['src_output'], d['bg_output'], d['context'], d['background'], d['background_map'],
                     d['init_state'])
         return eng

@@ -37,6 +37,8 @@ extern "C" {
 #define CASE_MAX_T 128
 #define CASE_MAX_SPLIT 16   /* additive-attention key splits */
 #define CASE_MAX_XSPLIT 64  /* cross-attention partials per (row, head) */
+#define CASE_MAX_BAN_SEQ 256 /* banned sequences of length >= 2 (case_tail_args_t.ban_tok rows) */
+#define CASE_MAX_BAN_LEN 16  /* tokens per banned sequence (case_tail_args_t.ban_tok columns) */
 
 #define CASE_F32 0
 #define CASE_BF16 1
@@ -418,6 +420,19 @@ typedef struct {
   const int32_t* hist_anc;
   int32_t hist_ld, t, eos;
   int32_t no_repeat_ngram, min_len;
+  /* case_sparse_tail only: banned words (all four or none; NULL = off).  Like the constraints above they need the answer
+   * history (hist_tok, hist_anc, hist_ld, t) and remove ids from the candidate set without renormalising; the banned set
+   * of a row is the union of every rule.
+   *   ban_mask: uint32 [ceil(V / 32)], bit (id & 31) of word id >> 5 set = id (0 <= id < V) is never a candidate.
+   *   ban_tok [CASE_MAX_BAN_SEQ][CASE_MAX_BAN_LEN], ban_len [CASE_MAX_BAN_SEQ], *ban_n = the number of sequences:
+   *     sequence i = (w_1 .. w_L), L = ban_len[i], bans w_L at step t when t >= L - 1 and y_{t-L+2} .. y_t == w_1 .. w_{L-1}.
+   * The content is read on the device at every launch (a captured graph serves every list): *ban_n is clamped to
+   * [0, CASE_MAX_BAN_SEQ] and a sequence whose length lies outside [2, CASE_MAX_BAN_LEN] is skipped.  The caller keeps the
+   * ids in [0, V) and at least 2K + hist_ld allowed ids per step: V - (ids of ban_mask) >= 2K + hist_ld + *ban_n. */
+  const uint32_t* ban_mask;
+  const int32_t* ban_tok;
+  const int32_t* ban_len;
+  const int32_t* ban_n;
 } case_tail_args_t;
 int case_row_tail(const case_tail_args_t* a, case_stream_t stream);
 int case_row_tail_max_vocab(void);
@@ -623,6 +638,12 @@ typedef struct {
    * would not take it (as for attribution), in CASE_MODE_MODULE_GREEDY, or with V < 2W + Tmax + 1 is refused before the
    * first launch; the n-best and attribution refusals come first. */
   int32_t no_repeat_ngram, min_len;
+  /* banned words (case_tail_args_t.ban_*; all four or none, NULL = off), same modes and the same sparse-tail requirement
+   * as the constraints: a request on a step that cannot serve it, with only some of the four pointers, or with
+   * V < 2W + Tmax + 1 is refused before the first launch, after the n-best, attribution and constraint checks.  The list
+   * lives in device memory and is read at every launch, so the caller enforces its content limits (ids in [0, V), at
+   * most CASE_MAX_BAN_SEQ sequences of 2 .. CASE_MAX_BAN_LEN tokens, V - (masked ids) >= 2W + Tmax + 1 + *ban_n). */
+  const uint32_t* ban_mask; const int32_t* ban_tok; const int32_t* ban_len; const int32_t* ban_n;
 } case_step_args_t;
 
 /* Enqueue one full decode step t (embedding .. select) for all R rows: the body of the eval loop
@@ -661,6 +682,8 @@ typedef struct {
    * first launch unless the step takes the sparse tail */
   case_attr_t* attr_cand; case_attr_t* attr_hist; case_attr_t* out_attr;
   int32_t no_repeat_ngram, min_len;                      /* search constraints (as in case_step_args_t) */
+  /* banned words (as in case_step_args_t) */
+  const uint32_t* ban_mask; const int32_t* ban_tok; const int32_t* ban_len; const int32_t* ban_n;
 } gttp_step_args_t;
 
 /* One GTTP decode step (GTTP/Model.py:176-193 -> BBCDecoder.forward :113-131 ->
